@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — headline benchmark of the B200-native Ed25519 / X25519 batch engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch-log2 20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch-log2 20] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): Ed25519 verify/s, sign/s & X25519 ops/s, batch 2^20 per GPU.
@@ -154,6 +154,16 @@ def synth_inputs(n, seed):
     return sec, msgs, pts
 
 
+DUMP_ROWS = 1 << 16          # rows of every output written by --dump-outputs: 16 MiB of signatures, 41.5 MiB in all
+
+
+def dump_rows(n):
+    """The rows --dump-outputs writes: all of them for small batches, else a fixed seeded sample (the same in every run)."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0x5EED00D0).choice(n, DUMP_ROWS, replace=False))
+
+
 # ---------------------------------------------------------------------------------------------------
 # reference arm: the reference's own CPU implementation on the host cores
 # ---------------------------------------------------------------------------------------------------
@@ -268,6 +278,15 @@ def run_ours(args):
         "x25519_base": lambda: ed.x25519_base_batch_dev(d_out, d_sec),
     }
 
+    rows = dump_rows(n) if args.dump_outputs and rank == 0 else None
+    outputs = {}
+
+    def keep(name, a):
+        """For --dump-outputs: the sampled rows of what the last timed step of a pass returned, as float32."""
+        if rows is not None:
+            a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+            outputs[name] = a[rows].astype(np.float32)
+
     from libeddsa_b200 import sharding
 
     def barrier():
@@ -300,14 +319,17 @@ def run_ours(args):
         sampler.start()
     launches0 = ed.launch_count()
     total_ms, per = timed(passes["verify"], K, W)
+    keep("verify", d_ok)
     launches = (ed.launch_count() - launches0) * K // (K + W)       # kernels launched by the K timed passes
     assert bool(d_ok.all().item()), "verify rejected a valid signature"
     value = world * n * K / (total_ms * 1e-3)
     kernel_ms = statistics.mean(per)
 
     also = {}
+    results = {"sign": d_sig, "x25519": d_out, "genpub": d_pub, "x25519_base": d_out}
     for name in ("sign", "x25519", "genpub", "x25519_base"):
         ms, p = timed(passes[name], K, W)
+        keep(name, results[name])
         rate = world * n * K / (ms * 1e-3)
         per_gpu = rate / world
         also[name] = {"value": rate, "unit": UNIT, "ms_per_step": ms / K,
@@ -343,11 +365,11 @@ def run_ours(args):
         dist.all_gather(t_all, torch.tensor([own_s], dtype=torch.float64, device=dev))
         per_rank = [float(t.item()) for t in t_all]
     assert bool(h_ok.all().item())
+    keep("e2e", h_ok)
     e2e_value = world * n * K / e2e_s
     # ---- the same from ordinary (pageable) memory: the library stages through its pinned slots ------------------
     p_sig, p_pub, p_msg, p_ok = np.array(h_sig.numpy()), np.array(h_pub.numpy()), np.array(h_msg.numpy()), np.empty(n, np.uint8)
     ap = lambda a: ctypes.c_void_p(a.ctypes.data)
-    Kx = min(K, 5)
 
     def e2e_pageable_step():
         rc = L.ed25519_verify_batch(n, ap(p_ok), ap(p_sig), ap(p_pub), ap(p_msg), None, 64)
@@ -364,10 +386,11 @@ def run_ours(args):
         barrier()
         return max_over_ranks(time.perf_counter() - t0)
 
-    pg_s = wall(e2e_pageable_step, Kx, 1)
+    pg_s = wall(e2e_pageable_step, K, 1)
     assert p_ok.all()
-    also["e2e_pageable"] = {"value": world * n * Kx / pg_s, "unit": UNIT, "api": "ed25519_verify_batch, ordinary (malloc) host buffers: staged through the "
-                            "library's pinned slots with memcpy", "ms_per_step": pg_s / Kx * 1e3}
+    keep("e2e_pageable", p_ok)
+    also["e2e_pageable"] = {"value": world * n * K / pg_s, "unit": UNIT, "api": "ed25519_verify_batch, ordinary (malloc) host buffers: staged through the "
+                            "library's pinned slots with memcpy", "ms_per_step": pg_s / K * 1e3}
     del p_sig, p_pub, p_msg
 
     # ---- BASELINE config 5's shape end to end: 1 KB messages, 10 % corrupted, pinned host buffers ----------------
@@ -390,11 +413,12 @@ def run_ours(args):
         if rc:
             raise RuntimeError(f"ed25519_verify_batch failed: {rc} {L.eddsa_b200_last_error()}")
 
-    kb_s = wall(e2e_1kb_step, Kx, 1)
+    kb_s = wall(e2e_1kb_step, K, 1)
     assert int(h_ok.sum().item()) == n - len(bad)
+    keep("e2e_1kb", h_ok)
     kb_bytes = n * (64 + 32 + mlen)
-    also["e2e_1kb"] = {"value": world * n * Kx / kb_s, "unit": UNIT, "api": "ed25519_verify_batch (host buffers, pinned), 1024-byte messages, 10 % of the signatures corrupted",
-                       "ms_per_step": kb_s / Kx * 1e3, "h2d_bytes_per_step": kb_bytes, "h2d_gbs_per_gpu": kb_bytes * Kx / kb_s / 1e9,
+    also["e2e_1kb"] = {"value": world * n * K / kb_s, "unit": UNIT, "api": "ed25519_verify_batch (host buffers, pinned), 1024-byte messages, 10 % of the signatures corrupted",
+                       "ms_per_step": kb_s / K * 1e3, "h2d_bytes_per_step": kb_bytes, "h2d_gbs_per_gpu": kb_bytes * K / kb_s / 1e9,
                        "note": "copy-bound: every signature brings 1 120 bytes over PCIe; compare h2d_gbs_per_gpu with also.inproc.copy_bandwidth"}
     del h_msg1k, h_sig1k
     clocks = sampler.stop() if rank == 0 else None
@@ -413,7 +437,7 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
     if rank == 0 and not args.no_inproc:
-        also["inproc"] = run_inproc(world)
+        also["inproc"] = run_inproc(world, K)
     if world > 1:
         dist.barrier(group=gloo)
 
@@ -462,6 +486,11 @@ def run_ours(args):
             "gpu_launches": int(launches),
             "roofline": roofline, "cpu_baseline": cpu_b, "also": also, "clocks": clocks,
         }
+        if rows is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "rows.npy"), rows.astype(np.float64))
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -505,10 +534,11 @@ def single_op_latency(ed, sec, pub, sig, msg, pts, calls=300):
     return res
 
 
-def run_inproc(world):
-    cmd = [sys.executable, os.path.join(ROOT, "tools", "inproc_bench.py"), "--devices", str(world)]
+def run_inproc(world, reps):
+    cmd = [sys.executable, os.path.join(ROOT, "tools", "inproc_bench.py"), "--devices", str(world), "--reps", str(reps)]
     drop = ("RANK", "WORLD_SIZE", "LOCAL_RANK", "LOCAL_WORLD_SIZE", "GROUP_RANK", "MASTER_ADDR", "MASTER_PORT", "EDDSA_B200_DEVICES", "OMP_NUM_THREADS")
     env = {k: v for k, v in os.environ.items() if k not in drop and not k.startswith("TORCHELASTIC")}
+    env["PYTHONDONTWRITEBYTECODE"] = "1"
     try:
         res = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=900)
         for line in reversed(res.stdout.strip().splitlines()):
@@ -552,6 +582,7 @@ def hbm_peak():
 
 
 def main():
+    sys.dont_write_bytecode = True       # the tree may be read-only: importing the package and the CPU checker writes nothing there
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -559,7 +590,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch-log2", type=int, default=20)
     ap.add_argument("--no-inproc", action="store_true", help="skip the in-library multi-device leg (configs 4 and 5 at 2^24)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step of each pass returned "
+                    "(rank 0, a fixed sample of rows) to DIR/<name>.npy as float32, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this project's GPU path (--impl ours)")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)
