@@ -88,7 +88,9 @@ EDDSA_DECL unsigned long long eddsa_b200_launch_count(void);
  * a, b, out are n x 32 little-endian bytes, any 256-bit values.  Used by the GPU unit tests. */
 EDDSA_DECL int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, int op);
 /* diagnostic: one operation modulo the group order L per item, executed by the device scalar library (op: 0
- * out = (a + 2^256 b) mod L, 1 out = a mod L, 2 out = a b + c mod L); a, b, c, out are n x 32 bytes. */
+ * out = (a + 2^256 b) mod L, 1 out = a mod L, 2 out = a b + c mod L, 3 out = tau and 4 out = |rho| (words 0..5;
+ * word 7: 1 if rho < 0) of the half-size verification scalars of t = a, 5 out = a recoded to the verify loop's
+ * signed 16-bit digits); a, b, c, out are n x 32 bytes. */
 EDDSA_DECL int eddsa_b200_sc_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *c, int op);
 /* diagnostic: copies the verify kernels' base-point window tables of the current device to `out`: table m (m = 0, 1)
  * holds e * 2^(128 m) * B for e = 0 .. 2^15 as 96-byte entries (y+x, y-x, 2dxy; canonical little-endian field

@@ -228,7 +228,9 @@ def peek_staging(which, slot, length):
 
 
 def sc_selftest(a, b, c, op):
-    """Diagnostic: scalar operation `op` (0 reduce512, 1 reduce256, 2 muladd) on n x 32-byte operands on the device."""
+    """Diagnostic: scalar operation `op` on n x 32-byte operands on the device: 0 (a + 2^256 b) mod L, 1 a mod L,
+    2 a b + c mod L, 3 tau and 4 |rho| (words 0..5; word 7 = 1 if rho < 0) of the half-size verification scalars of
+    t = a < L, 5 a < 2^253 recoded to the verify loop's signed 16-bit digits (a + 2^15 sum_k 2^(16 k))."""
     a, b, c = _arr(a, 32, "a"), _arr(b, 32, "b"), _arr(c, 32, "c")
     out = np.empty_like(a)
     _check(lib().eddsa_b200_sc_selftest(len(a), _p(out), _p(a), _p(b), _p(c), op), "eddsa_b200_sc_selftest")
@@ -330,3 +332,13 @@ def x25519_batch_dev(out, scalar, point):
 def x25519_base_batch_dev(out, scalar):
     n = scalar.numel() // 32
     _check(lib().x25519_base_batch_dev(n, _dp(out), _dp(scalar), _stream()), "x25519_base_batch_dev")
+
+
+def pk_ed25519_to_x25519_batch_dev(out, pk):
+    n = pk.numel() // 32
+    _check(lib().pk_ed25519_to_x25519_batch_dev(n, _dp(out), _dp(pk), _stream()), "pk_ed25519_to_x25519_batch_dev")
+
+
+def sk_ed25519_to_x25519_batch_dev(out, sk):
+    n = sk.numel() // 32
+    _check(lib().sk_ed25519_to_x25519_batch_dev(n, _dp(out), _dp(sk), _stream()), "sk_ed25519_to_x25519_batch_dev")

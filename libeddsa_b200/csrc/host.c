@@ -759,7 +759,9 @@ int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8
 }
 
 /* diagnostic: one scalar operation mod L per item on the device (op: 0 out = (a || b) mod L, the 64-byte value
- * a + 2^256 b; 1 out = a mod L; 2 out = a * b + c mod L); a, b, c, out: n x 32 bytes */
+ * a + 2^256 b; 1 out = a mod L; 2 out = a * b + c mod L; 3 out = tau of the half-size verification scalars
+ * (rho, tau) of t = a, a < L; 4 out = |rho| of the same in words 0..5, 1 in word 7 if rho < 0; 5 out = a + 2^15 sum
+ * 2^(16 k), the signed 16-bit digits of a < 2^253 as the verify loop reads them); a, b, c, out: n x 32 bytes */
 int eddsa_b200_sc_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *c, int op)
 {
     edg_job_t j = {OP_SC_TEST, n, 3, {a, b, c}, {32, 32, 32}, 0, NULL, NULL, (size_t)op, out, 32};

@@ -70,7 +70,9 @@ __global__ void __launch_bounds__(kThreads) k_fe_selftest(size_t n, uint8_t *out
     }
 }
 
-// op 0: out = (a + 2^256 b) mod L (sc_reduce512); 1: out = a mod L (sc_reduce256); 2: out = a b + c mod L (sc_muladd)
+// op 0: out = (a + 2^256 b) mod L (sc_reduce512); 1: out = a mod L (sc_reduce256); 2: out = a b + c mod L (sc_muladd);
+// 3: out = tau of half_gcd(t = a); 4: out = |rho| of half_gcd(t = a) in words 0..5, the sign of rho (rho_neg) in word 7;
+// 5: out = sc_recode_window(a), the signed 16-bit digits of rho S the verify loop reads
 __global__ void __launch_bounds__(kThreads) k_sc_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *c, int op) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         u32 x[16], z[8], r[8];
@@ -79,7 +81,14 @@ __global__ void __launch_bounds__(kThreads) k_sc_selftest(size_t n, uint8_t *out
         load8(z, c, i);
         if (op == 0) sc_reduce512(r, x);
         else if (op == 1) sc_reduce256(r, x);
-        else sc_muladd(r, x, x + 8, z);
+        else if (op == 3 || op == 4) {
+            u32 rho[8], tau[8], neg;
+            half_gcd(rho, neg, tau, x);
+            for (int w = 0; w < 8; w++) r[w] = op == 3 ? tau[w] : (w < 6 ? rho[w] : (w == 7 ? neg : 0u));
+        } else if (op == 5) {
+            for (int w = 0; w < 8; w++) r[w] = x[w];
+            sc_recode_window(r);
+        } else sc_muladd(r, x, x + 8, z);
         store8(out, i, r);
     }
 }

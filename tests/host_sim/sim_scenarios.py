@@ -1029,6 +1029,48 @@ def scenario_real_kernels_full_scalars():
     sim.clean()
 
 
+def scenario_real_kernels_structured():
+    """The rare branches of the scalar code on the real kernels, checked against Python integers and the CPU reference (never
+    against another build of the same headers): half_gcd (k_sc_selftest ops 3 and 4) on structured challenges that reach every
+    branch class of tests/structured_inputs.py, the verify loop's 16-bit recoding (op 5) on digit-run values, and x25519_base
+    (k_comb<1>: signed radix-64 recoding + tensor-core lookup) on scalars whose clamped value mod L has structured digits."""
+    import structured_inputs as si
+    from cpu_ref import best_cpu_impl
+    assert "sim_kernels" in SIM_SO
+    sim, cpu = Sim(), best_cpu_impl()
+    ed = sim.ed
+    rows = lambda vals: np.frombuffer(b"".join(v.to_bytes(32, "little") for v in vals), np.uint8).reshape(-1, 32)
+    val = lambda a: [int.from_bytes(a[i].tobytes(), "little") for i in range(len(a))]
+    ts = si.half_gcd_inputs()
+    counts = si.class_counts(ts)
+    print("half_gcd inputs by branch class:", counts)
+    assert all(counts[k] >= m for k, m in si.MIN_CLASS_COUNT.items()), counts
+    a = rows(ts)
+    z = np.zeros_like(a)
+    taus, rhos = val(ed.sc_selftest(a, z, z, 3)), ed.sc_selftest(a, z, z, 4)
+    for i, t in enumerate(ts):
+        want_r, want_ta, info = si.half_gcd_model(t)
+        w = rhos[i].view(np.uint32)
+        r = int.from_bytes(rhos[i, :24].tobytes(), "little")
+        assert w[6] == 0 and w[7] in (0, 1), (t, w)
+        r = -r if w[7] else r
+        assert (r, taus[i]) == (want_r, want_ta), (t, info, r, taus[i], want_r, want_ta)
+    xs = si.recode_window_values(n_random=300)
+    es = val(ed.sc_selftest(rows(xs), np.zeros((len(xs), 32), np.uint8), np.zeros((len(xs), 32), np.uint8), 5))
+    for x, e in zip(xs, es):
+        ds = si.window_digits(e)
+        assert all(-2**15 <= d < 2**15 for d in ds) and sum(d << (16 * k) for k, d in enumerate(ds)) == x, (x, e)
+    scal, targets, unreachable = si.comb_batch(n_random=300)
+    print(f"comb targets: {sum(t is not None for t in targets)} reachable through x25519_base, {unreachable} dropped")
+    sa = np.frombuffer(b"".join(scal), np.uint8).reshape(-1, 32)
+    got = ed.x25519_base_batch(sa)
+    eq(got, cpu.x25519_base(sa), "x25519_base with structured comb digits, against the CPU reference")
+    picked = [i for i, t in enumerate(targets) if t is not None][:25]
+    for i in picked:
+        assert got[i].tobytes() == si.x25519_base_model(targets[i]), (i, targets[i])
+    sim.clean()
+
+
 def scenario_real_kernels_opcount():
     """Field operations the REAL verify kernels execute per signature, counted by the emulator (a lane of the loop kernel runs its
     warp's maximum window count, as on the device): the figure the integer-multiply roofline of bench.py is computed from."""

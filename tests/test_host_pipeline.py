@@ -85,7 +85,8 @@ SCENARIOS = {
 KERNELS_SO = os.path.join(HS, "libeddsa_sim_kernels.so")
 # (the all_ops and lifecycle scenarios and the other stream schedules pass on it too; left out of the suite for time: ~30 s each)
 REAL_KERNEL_RUNS = [("real_kernels", {"CUDASIM_DEVICES": "1", "EDDSA_B200_VERIFY_WAVES": "1"}),
-                    ("real_kernels_full_scalars", {"CUDASIM_DEVICES": "1", "EDDSA_B200_DEBUG_FULL_SCALARS": "1"})]
+                    ("real_kernels_full_scalars", {"CUDASIM_DEVICES": "1", "EDDSA_B200_DEBUG_FULL_SCALARS": "1"}),
+                    ("real_kernels_structured", {"CUDASIM_DEVICES": "1"})]
 
 OTHER_SCHEDULES = [(n, sch) for n in ("chunks", "budget", "multi", "threads", "dev_api", "failures") for sch in ("others-first", "eager", "random")
                    if n != "failures" or sch == "others-first"]        # the failure sweep: the two adversarial schedules only (12 s each)

@@ -284,29 +284,38 @@ def test_tensor_core_lookup_layout(ops):
 
 def test_half_gcd(ops):
     """hgcd.cuh: (rho, tau) is a lattice vector (tau = rho t mod 8L), rho is odd, and both are short — for random t,
-    for structured t (tiny, huge partial quotients, even-rho traps) and for the documented fallback."""
-    L = 2**252 + 27742317777372353535851937790883648493
+    for structured t (tiny, huge partial quotients, even-rho traps) and for the documented fallback.  Beyond these
+    invariants the result is deterministic: it must be exactly the vector a plain extended Euclid on (8L, t) stops at
+    (tests/structured_inputs.py: half_gcd_model).  The structured challenges place partial quotients of 2^16 - 1 .. 2^64 at
+    chosen continued-fraction depths, so that every rare branch (no Lehmer step, the word-shift loop, the large quotient
+    across 2^128, even rho, the rv < 2^96 fallback) is taken a minimum number of times."""
+    import structured_inputs as si
     N = 8 * L
-    rng = random.Random(11)
-    ts = [0, 1, 2, 3, 5, 2**127, 2**128 - 1, 2**128, 2**128 + 1, L - 1, L - 2, (N + 1) // 2 % L, (L + 1) // 2, L // 3, L // 5,
-          2**200, 2**252, 2**251 + 7, (1 << 129) + 1, N // (2**64 + 13) % L, pow(3, -1, N) % L, pow(5, -1, N) % L,
-          pow(2**64 + 1, -1, N) % L, pow(2**126 + 1, -1, N) % L, pow(2**130 + 3, -1, N) % L]
-    ts += [rng.getrandbits(k) % L for k in (16, 64, 100, 128, 129, 160, 200, 252) for _ in range(40)]
-    ts += [rng.randrange(L) for _ in range(3000)]
+    legacy = si.half_gcd_legacy_ts()
+    ts = si.half_gcd_inputs()
+    counts = si.class_counts(ts)
+    print("half_gcd inputs by branch class:", counts)
+    assert all(counts[k] >= m for k, m in si.MIN_CLASS_COUNT.items()), counts
     rho = (ctypes.c_uint32 * 8)(); tau = (ctypes.c_uint32 * 8)(); neg = ctypes.c_uint32()
     worst = 0; falls = 0
+    legacy_set = set(legacy)
     for t in ts:
         tw = (ctypes.c_uint32 * 8)(*[(t >> (32 * i)) & 0xffffffff for i in range(8)])
         ops.hs_half_gcd(rho, ctypes.byref(neg), tau, tw)
         r = sum(int(rho[i]) << (32 * i) for i in range(8)); ta = sum(int(tau[i]) << (32 * i) for i in range(8))
+        assert rho[6] == 0 and rho[7] == 0 and neg.value in (0, 1), t
         r = -r if neg.value else r
         assert r % 2 == 1, (t, r)
         assert (r * t - ta) % N == 0, (t, r, ta)
-        if abs(r) == 1 and ta == t and t >= 2**128:
-            falls += 1                                   # fallback (rho, tau) = (1, t): allowed, must be rare
+        want_r, want_ta, info = si.half_gcd_model(t)
+        assert (r, ta) == (want_r, want_ta), (t, r, ta, want_r, want_ta, info)
+        if info["fallback"]:
+            assert (r, ta) == (1, t)
+            falls += t in legacy_set                     # fallback (rho, tau) = (1, t): allowed, must be rare
         else:
             assert ta < 2**128 and abs(r) < 2**160, (t, r, ta)
-            worst = max(worst, abs(r).bit_length(), ta.bit_length())
+            if t in legacy_set:
+                worst = max(worst, abs(r).bit_length(), ta.bit_length())
     assert falls <= 10, falls                      # only structured t (short even vectors such as t = L - 1) may fall back
     assert worst <= 150, worst
 
