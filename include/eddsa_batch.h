@@ -84,7 +84,8 @@ EDDSA_DECL int eddsa_b200_set_device_count(int count);
 EDDSA_DECL unsigned long long eddsa_b200_launch_count(void);
 /* diagnostic: one GF(2^255-19) operation per item, executed by the device field library (op: 0 mul,
  * 1 square, 2 add, 3 sub, 4 times 121665, 5 canonical form, 6 inverse, 7 power (p-5)/8, 8 negate,
- * 9 the kernels' shared inversion over each group of 32 consecutive items of a, 0 -> 0);
+ * 9 the kernels' shared inversion over each group of 32 consecutive items of a, 0 -> 0; 10 .. 15 the
+ * public-data flavour the verify kernels use of ops 0, 1, 2, 3, 8, 7, with results identical to those ops);
  * a, b, out are n x 32 little-endian bytes, any 256-bit values.  Used by the GPU unit tests. */
 EDDSA_DECL int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, int op);
 /* diagnostic: one operation modulo the group order L per item, executed by the device scalar library (op: 0

@@ -255,12 +255,22 @@ static inline u32 subw8(u32 r[8], u32 x) {
 // lives in, so ptxas never has to re-pair registers with moves.
 
 // last step shared by both: w[0..7] + 38 * t8 (t8 <= 40) -> r; if that wraps past 2^256 the wrapped value is
-// tiny, so the final +38 cannot carry again
-__device__ __forceinline__ void fe_fold_tail(fe &r, u32 *w, u32 t8) {
-    const u32 c2 = addw8(w, t8 * 38u);
-    r.v[0] = w[0] + (38u & (0u - c2));
+// tiny, so the final +38 cannot carry again.  PUB (public data only): word 0 alone, returns the pending carry
+// into word 1 (see pub_settle_add below).
+template <bool PUB> __device__ __forceinline__ bool fe_fold_tail(fe &r, u32 *w, u32 t8) {
+    if constexpr (PUB) {
+        const u32 x = t8 * 38u;
+        r.v[0] = w[0] + x;
 #pragma unroll
-    for (int j = 1; j < 8; j++) r.v[j] = w[j];
+        for (int j = 1; j < 8; j++) r.v[j] = w[j];
+        return r.v[0] < x;
+    } else {
+        const u32 c2 = addw8(w, t8 * 38u);
+        r.v[0] = w[0] + (38u & (0u - c2));
+#pragma unroll
+        for (int j = 1; j < 8; j++) r.v[j] = w[j];
+        return false;
+    }
 }
 
 // words 0..7 += 38 * (even words of the high half); returns the carry out
@@ -275,7 +285,7 @@ __device__ __forceinline__ u32 fe_fold_even(u32 *w) {
 }
 
 // Multiplication: even-word accumulator w[0..15], odd-word accumulator od[0..14] (od[k] = word k + 1), not yet merged.
-__device__ __forceinline__ void fe_fold_mul(fe &r, u32 *w, u32 *od) {
+template <bool PUB> __device__ __forceinline__ bool fe_fold_mul(fe &r, u32 *w, u32 *od) {
     // high half first: words 8..15 += od[7..14] (the product is < 2^512: no carry out)
     asm("add.cc.u32 %0, %0, %8; addc.cc.u32 %1, %1, %9; addc.cc.u32 %2, %2, %10; addc.cc.u32 %3, %3, %11; "
         "addc.cc.u32 %4, %4, %12; addc.cc.u32 %5, %5, %13; addc.cc.u32 %6, %6, %14; addc.u32 %7, %7, %15;"
@@ -293,12 +303,12 @@ __device__ __forceinline__ void fe_fold_mul(fe &r, u32 *w, u32 *od) {
         "addc.cc.u32 %4, %4, %12; addc.cc.u32 %5, %5, %13; addc.cc.u32 %6, %6, %14; addc.u32 %7, %7, %15;"
         : "+r"(w[1]), "+r"(w[2]), "+r"(w[3]), "+r"(w[4]), "+r"(w[5]), "+r"(w[6]), "+r"(w[7]), "+r"(t8)
         : "r"(od[0]), "r"(od[1]), "r"(od[2]), "r"(od[3]), "r"(od[4]), "r"(od[5]), "r"(od[6]), "r"(x));
-    fe_fold_tail(r, w, t8);
+    return fe_fold_tail<PUB>(r, w, t8);
 }
 
 // Squaring: one merged 16-word value w.  The odd high words are multiplied without a chain (their register
 // pairs would be misaligned against w) and added in with one carry chain.
-__device__ __forceinline__ void fe_fold_sq(fe &r, u32 *w) {
+template <bool PUB> __device__ __forceinline__ bool fe_fold_sq(fe &r, u32 *w) {
     u32 t8 = fe_fold_even(w);
     const u64 q0 = mulw(w[9], 38u), q1 = mulw(w[11], 38u), q2 = mulw(w[13], 38u), q3 = mulw(w[15], 38u);
     asm("add.cc.u32 %0, %0, %8; addc.cc.u32 %1, %1, %9; addc.cc.u32 %2, %2, %10; addc.cc.u32 %3, %3, %11; "
@@ -306,39 +316,117 @@ __device__ __forceinline__ void fe_fold_sq(fe &r, u32 *w) {
         : "+r"(w[1]), "+r"(w[2]), "+r"(w[3]), "+r"(w[4]), "+r"(w[5]), "+r"(w[6]), "+r"(w[7]), "+r"(t8)
         : "r"((u32)q0), "r"((u32)(q0 >> 32)), "r"((u32)q1), "r"((u32)(q1 >> 32)), "r"((u32)q2), "r"((u32)(q2 >> 32)),
           "r"((u32)q3), "r"((u32)(q3 >> 32)));
-    fe_fold_tail(r, w, t8);
+    return fe_fold_tail<PUB>(r, w, t8);
 }
 #else
-static inline void fe_fold512(fe &r, const u32 w[17]) {
+template <bool PUB> static inline bool fe_fold512(fe &r, const u32 w[17]) {
     u64 c = 0;
     for (int j = 0; j < 8; j++) {
         const u64 t = mulw(w[8 + j], 38u) + w[j] + c;
         r.v[j] = (u32)t;
         c = t >> 32;
     }
+    if (PUB) {
+        const u32 x = (u32)c * 38u;
+        r.v[0] += x;
+        return r.v[0] < x;
+    }
     const u32 c2 = addw8(r.v, (u32)c * 38u);
     r.v[0] += 38u & (0u - c2);
+    return false;
 }
 #endif
 
+// Two flavours of every operation that ends in a fold (2^256 = 38 mod p, i.e. a small value added into an 8-word
+// value and carried through all eight words):
+//   * PUB = false, the names fe_add, fe_sub, fe_mul, .. : the full carry chain, always.  Constant time; the only
+//     form the secret-key kernels use.
+//   * PUB = true, the names pub_add, pub_sub, pub_mul, .. : the fold is added into word 0 only, and the carry (or
+//     borrow) out of word 0 is RETURNED as a pending flag instead of being carried on.  The caller computes a group of
+//     independent operations, ORs their flags and, only if one is set, settles the affected results with
+//     pub_settle_add / pub_settle_sub, which finish exactly the chain the constant-time form runs.  Results are
+//     therefore bit-identical to the constant-time forms for every input.  A flag is set only when word 0 ends within
+//     1520 of 2^32 (below 4e-7 per operation on data that is not crafted), so the rare path costs nothing on average,
+//     but whether it runs depends on the operands: for public data only (verification, public-key conversion).
 // r = a + b                                            [reference: fld_add, fld.h:94]
-EDG_HD void fe_add(fe &r, const fe &a, const fe &b) {
+template <bool PUB> EDG_HD bool fe_add_t(fe &r, const fe &a, const fe &b) {
     u32 t[8];
     const u32 c = add8(t, a.v, b.v);
-    const u32 c2 = addw8(t, 38u & (0u - c));           // 2^256 = 38 (mod p)
-    t[0] += 38u & (0u - c2);
+    bool pend = false;
+    if (PUB) {
+        const u32 x = 38u & (0u - c);                   // 2^256 = 38 (mod p)
+        t[0] += x;
+        pend = t[0] < x;
+    } else {
+        const u32 c2 = addw8(t, 38u & (0u - c));
+        t[0] += 38u & (0u - c2);
+    }
 #pragma unroll
     for (int i = 0; i < 8; i++) r.v[i] = t[i];
+    return pend;
 }
 
 // r = a - b                                            [reference: fld_sub, fld.h:102]
-EDG_HD void fe_sub(fe &r, const fe &a, const fe &b) {
+template <bool PUB> EDG_HD bool fe_sub_t(fe &r, const fe &a, const fe &b) {
     u32 t[8];
     const u32 bw = sub8(t, a.v, b.v);                   // borrow: t = a - b + 2^256, so take 38 off again
-    const u32 bw2 = subw8(t, 38u & bw);
-    t[0] -= 38u & bw2;
+    bool pend = false;
+    if (PUB) {
+        const u32 x = 38u & bw;
+        pend = t[0] < x;
+        t[0] -= x;
+    } else {
+        const u32 bw2 = subw8(t, 38u & bw);
+        t[0] -= 38u & bw2;
+    }
 #pragma unroll
     for (int i = 0; i < 8; i++) r.v[i] = t[i];
+    return pend;
+}
+
+EDG_HD void fe_add(fe &r, const fe &a, const fe &b) { fe_add_t<false>(r, a, b); }
+EDG_HD void fe_sub(fe &r, const fe &a, const fe &b) { fe_sub_t<false>(r, a, b); }
+EDG_HD bool pub_add(fe &r, const fe &a, const fe &b) { return fe_add_t<true>(r, a, b); }
+EDG_HD bool pub_sub(fe &r, const fe &a, const fe &b) { return fe_sub_t<true>(r, a, b); }
+EDG_HD bool pub_dbl(fe &r, const fe &a) { return fe_add_t<true>(r, a, a); }
+EDG_HD bool pub_neg(fe &r, const fe &a) {
+    fe z;
+    fe_set_u32(z, 0);
+    return fe_sub_t<true>(r, z, a);
+}
+
+// The rare path of the public flavour: r came from a pub_ operation that returned pend.  Carry (borrow) the pending
+// 1 through words 1..7 and, if it leaves word 7, add (take off) the second 38 — the rest of the constant-time chain.
+EDG_HD void pub_settle_add(fe &r, bool pend) {
+    if (!pend) return;
+    u32 t[8];
+#pragma unroll
+    for (int i = 0; i < 7; i++) t[i] = r.v[i + 1];
+    t[7] = 0;
+    addw8(t, 1u);                                       // t[7] = carry out of word 7
+#pragma unroll
+    for (int i = 0; i < 7; i++) r.v[i + 1] = t[i];
+    r.v[0] += 38u & (0u - t[7]);
+}
+EDG_HD void pub_settle_sub(fe &r, bool pend) {
+    if (!pend) return;
+    u32 t[8];
+#pragma unroll
+    for (int i = 0; i < 7; i++) t[i] = r.v[i + 1];
+    t[7] = 0;
+    subw8(t, 1u);                                       // t[7] = borrow out of word 7 as a mask
+#pragma unroll
+    for (int i = 0; i < 7; i++) r.v[i + 1] = t[i];
+    r.v[0] -= 38u & t[7];
+}
+
+// branch hint for the OR of a group's pending flags
+EDG_HD bool pub_rare(bool pend) {
+#if defined(__CUDACC__) || defined(__GNUC__)
+    return __builtin_expect(pend != 0, 0);
+#else
+    return pend != 0;
+#endif
 }
 
 // r = -a                                               [reference: fld_neg, fld.h:138]
@@ -352,7 +440,7 @@ EDG_HD void fe_neg(fe &r, const fe &a) {
 EDG_HD void fe_dbl(fe &r, const fe &a) { fe_add(r, a, a); }
 
 // r = a * b mod p.  72 IMAD.WIDE.U32.                            [reference: fld_mul, fld.c:210 / :448]
-EDG_FE_MUL void fe_mul(fe &r, const fe &a, const fe &b) {
+template <bool PUB> EDG_FE_MUL bool fe_mul_t(fe &r, const fe &a, const fe &b) {
     EDG_COUNT_MUL();
     u32 w[17];
 #if defined(__CUDA_ARCH__)
@@ -371,7 +459,7 @@ EDG_FE_MUL void fe_mul(fe &r, const fe &a, const fe &b) {
             cmad<4>(od + i - 1, a.v, b.v[i]);
         }
     }
-    fe_fold_mul(r, w, od);
+    return fe_fold_mul<PUB>(r, w, od);
 #else
     for (int i = 0; i < 17; i++) w[i] = 0;
     for (int i = 0; i < 8; i++) {
@@ -379,13 +467,13 @@ EDG_FE_MUL void fe_mul(fe &r, const fe &a, const fe &b) {
         for (int j = 0; j < 8; j++) { const u64 t = mulw(a.v[j], b.v[i]) + w[i + j] + c; w[i + j] = (u32)t; c = t >> 32; }
         w[i + 8] = (u32)c;
     }
-    fe_fold512(r, w);
+    return fe_fold512<PUB>(r, w);
 #endif
 }
 
 // r = a^2 mod p.  44 IMAD.WIDE.U32 (28 cross products, doubled by a 1-bit shift, + 8 squares + 8 fold).
 //                                                                  [reference: fld_sq, fld.c:250 / :503]
-EDG_FE_MUL void fe_sq(fe &r, const fe &a) {
+template <bool PUB> EDG_FE_MUL bool fe_sq_t(fe &r, const fe &a) {
     EDG_COUNT_SQ();
     u32 w[17];
 #if defined(__CUDA_ARCH__)
@@ -411,7 +499,7 @@ EDG_FE_MUL void fe_sq(fe &r, const fe &a) {
     for (int k = 15; k > 0; k--) w[k] = (w[k] << 1) | (w[k - 1] >> 31);        // x2 (word 0 holds no cross product)
     w[0] = 0;
     add_squares(w, a.v);
-    fe_fold_sq(r, w);
+    return fe_fold_sq<PUB>(r, w);
 #else
     for (int i = 0; i < 17; i++) w[i] = 0;
     for (int i = 0; i < 8; i++) {
@@ -419,8 +507,25 @@ EDG_FE_MUL void fe_sq(fe &r, const fe &a) {
         for (int j = 0; j < 8; j++) { const u64 t = mulw(a.v[j], a.v[i]) + w[i + j] + c; w[i + j] = (u32)t; c = t >> 32; }
         w[i + 8] = (u32)c;
     }
-    fe_fold512(r, w);
+    return fe_fold512<PUB>(r, w);
 #endif
+}
+
+EDG_HD void fe_mul(fe &r, const fe &a, const fe &b) { fe_mul_t<false>(r, a, b); }
+EDG_HD void fe_sq(fe &r, const fe &a) { fe_sq_t<false>(r, a); }
+EDG_HD bool pub_mul(fe &r, const fe &a, const fe &b) { return fe_mul_t<true>(r, a, b); }
+EDG_HD bool pub_sq(fe &r, const fe &a) { return fe_sq_t<true>(r, a); }
+
+// One operation of either flavour, settled at once (a group of one), for code shared by both: with PUB = false the
+// flag is the constant false and these are exactly fe_mul, fe_sq, fe_add, fe_sub.
+template <bool PUB> EDG_HD void fe_mul_s(fe &r, const fe &a, const fe &b) { const bool p = fe_mul_t<PUB>(r, a, b); if (pub_rare(p)) pub_settle_add(r, p); }
+template <bool PUB> EDG_HD void fe_sq_s(fe &r, const fe &a) { const bool p = fe_sq_t<PUB>(r, a); if (pub_rare(p)) pub_settle_add(r, p); }
+template <bool PUB> EDG_HD void fe_add_s(fe &r, const fe &a, const fe &b) { const bool p = fe_add_t<PUB>(r, a, b); if (pub_rare(p)) pub_settle_add(r, p); }
+template <bool PUB> EDG_HD void fe_sub_s(fe &r, const fe &a, const fe &b) { const bool p = fe_sub_t<PUB>(r, a, b); if (pub_rare(p)) pub_settle_sub(r, p); }
+template <bool PUB> EDG_HD void fe_neg_s(fe &r, const fe &a) {
+    fe z;
+    fe_set_u32(z, 0);
+    fe_sub_s<PUB>(r, z, a);
 }
 
 // r = a * 121665 mod p.                     [reference: fld_scale, fld.c:184/:430; only s = 121665 is used, x25519.c:77]
@@ -536,9 +641,9 @@ EDG_HD void fe_cswap(fe &a, fe &b, u32 mask) {
 // compact, table-driven routine so that a kernel carries a single copy of the chain instead of ~20
 // inlined multiplies (instruction-cache footprint; the chain is 254 S + 11 M / 251 S + 11 M exactly as
 // in the reference).  Program step: acc = acc^(2^n) * S[m] (m = 4: no multiply), then S[st] = acc
-// (st = 4: no store).  Control flow depends only on these public constants.
+// (st = 4: no store).  Control flow depends only on these public constants (and, with PUB, on the public z).
 //                                                           [reference: fld_inv fld.c:579-645, fld_pow2523 fld.c:658-709]
-EDG_POW_INLINE void fe_pow_chain(fe *out, const fe *zin, int which) {
+template <bool PUB> EDG_POW_INLINE void fe_pow_chain(fe *out, const fe *zin, int which) {
     // program packed into immediates (no table in local memory):     step: 0   1   2    3   4    5    6    7    8     9    10   11
     //   squarings n                                                         1   2   0    1   5   10   20   10   50   100   50   (5|2)
     //   multiplier slot m (4 = none)                                         4   0   1    2   2    2    3    2    2     3    2   (1|0)
@@ -557,11 +662,11 @@ EDG_POW_INLINE void fe_pow_chain(fe *out, const fe *zin, int which) {
         const int st = (int)((PROG_S >> (4 * step)) & 0xf);
         if (step == 11) { n = which ? 5 : 2; m = which ? 1 : 0; }   // * z11 (inverse) or * z (pow2523)
 #pragma unroll 1
-        for (int i = 0; i < n; i++) fe_sq(acc, acc);
+        for (int i = 0; i < n; i++) fe_sq_s<PUB>(acc, acc);
         if (m != 4) {
             fe t;
             if (m == 0) fe_copy(t, s0); else if (m == 1) fe_copy(t, s1); else if (m == 2) fe_copy(t, s2); else fe_copy(t, s3);
-            fe_mul(acc, acc, t);
+            fe_mul_s<PUB>(acc, acc, t);
         }
         if (st == 1) fe_copy(s1, acc); else if (st == 2) fe_copy(s2, acc); else if (st == 3) fe_copy(s3, acc);
     }
@@ -569,9 +674,10 @@ EDG_POW_INLINE void fe_pow_chain(fe *out, const fe *zin, int which) {
 }
 
 // r = z^(p-2) = z^-1 (0 -> 0).  254 S + 11 M.                      [reference: fld_inv, fld.c:579]
-EDG_HD void fe_inv(fe &r, const fe &z) { fe_pow_chain(&r, &z, 1); }
+EDG_HD void fe_inv(fe &r, const fe &z) { fe_pow_chain<false>(&r, &z, 1); }
 
 // r = z^((p-5)/8) = z^(2^252 - 3).  251 S + 11 M.                  [reference: fld_pow2523, fld.c:658]
-EDG_HD void fe_pow2523(fe &r, const fe &z) { fe_pow_chain(&r, &z, 0); }
+EDG_HD void fe_pow2523(fe &r, const fe &z) { fe_pow_chain<false>(&r, &z, 0); }
+EDG_HD void pub_pow2523(fe &r, const fe &z) { fe_pow_chain<true>(&r, &z, 0); }
 
 }  // namespace edg

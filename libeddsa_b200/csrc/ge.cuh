@@ -64,31 +64,32 @@ EDG_HD void ge_madd(ge_p3 &r, const ge_p3 &p, const ge_pre &q, bool need_t) {
 }
 
 // r = p + q, q projective cached.  8M (7M when !need_t).                        [ed_add, ed.c:175]
-EDG_HD void ge_add_cached(ge_p3 &r, const ge_p3 &p, const ge_cached &q, bool need_t) {
+// PUB: the public-data flavour of the field operations (fe.cuh), for points that are public.
+template <bool PUB = false> EDG_HD void ge_add_cached(ge_p3 &r, const ge_p3 &p, const ge_cached &q, bool need_t) {
     fe a, b, c, d, e, f, g, h;
-    fe_sub(a, p.Y, p.X);
-    fe_mul(a, a, q.ymx);                
-    fe_add(b, p.Y, p.X);
-    fe_mul(b, b, q.ypx);                
-    fe_mul(c, p.T, q.t2d);              
-    fe_mul(d, p.Z, q.z2);               
-    fe_sub(e, b, a);
-    fe_sub(f, d, c);
-    fe_add(g, d, c);
-    fe_add(h, b, a);
-    fe_mul(r.X, e, f);
-    fe_mul(r.Y, g, h);
-    fe_mul(r.Z, f, g);
-    if (need_t) fe_mul(r.T, e, h);
+    fe_sub_s<PUB>(a, p.Y, p.X);
+    fe_mul_s<PUB>(a, a, q.ymx);                
+    fe_add_s<PUB>(b, p.Y, p.X);
+    fe_mul_s<PUB>(b, b, q.ypx);                
+    fe_mul_s<PUB>(c, p.T, q.t2d);              
+    fe_mul_s<PUB>(d, p.Z, q.z2);               
+    fe_sub_s<PUB>(e, b, a);
+    fe_sub_s<PUB>(f, d, c);
+    fe_add_s<PUB>(g, d, c);
+    fe_add_s<PUB>(h, b, a);
+    fe_mul_s<PUB>(r.X, e, f);
+    fe_mul_s<PUB>(r.Y, g, h);
+    fe_mul_s<PUB>(r.Z, f, g);
+    if (need_t) fe_mul_s<PUB>(r.T, e, h);
 }
 
 // cached form of p: Y+X, Y-X, 2Z, 2dT.      [ed_precompute, ed.c:436]
-EDG_HD void ge_to_cached(ge_cached &c, const ge_p3 &p) {
+template <bool PUB = false> EDG_HD void ge_to_cached(ge_cached &c, const ge_p3 &p) {
     const fe d2 = EDG_FE_2D;
-    fe_add(c.ypx, p.Y, p.X);
-    fe_sub(c.ymx, p.Y, p.X);
-    fe_dbl(c.z2, p.Z);
-    fe_mul(c.t2d, p.T, d2);
+    fe_add_s<PUB>(c.ypx, p.Y, p.X);
+    fe_sub_s<PUB>(c.ymx, p.Y, p.X);
+    fe_add_s<PUB>(c.z2, p.Z, p.Z);
+    fe_mul_s<PUB>(c.t2d, p.T, d2);
 }
 
 // cached point <-> 32 contiguous words of per-thread scratch (16-byte aligned): 8 x 128-bit accesses
@@ -116,14 +117,6 @@ EDG_HD void ge_cached_load(ge_cached &c, const u32 *src) {
 #endif
 #pragma unroll
     for (int i = 0; i < 8; i++) { c.ypx.v[i] = w[i]; c.ymx.v[i] = w[8 + i]; c.z2.v[i] = w[16 + i]; c.t2d.v[i] = w[24 + i]; }
-}
-
-// q = neg ? -q : q for a cached point, neg an all-ones/zero mask (public data in verify, but branch-free anyway)
-EDG_HD void ge_cached_cneg(ge_cached &q, u32 neg) {
-    fe_cswap(q.ypx, q.ymx, neg);
-    fe nt;
-    fe_neg(nt, q.t2d);
-    fe_select(q.t2d, q.t2d, nt, neg);
 }
 
 // q = neg ? -q : q for an affine precomputed point (canonical limbs).           [scale16, ed.c:384-390]
@@ -267,9 +260,10 @@ __device__ __forceinline__ void ge_pre_select_mma(ge_pre &t, const u32 *row_mma,
 // reference: bit 255 is the sign, the low 255 bits are y and are NOT range-checked (y >= p is
 // reduced), x = 0 with sign 1 stays 0.  Returns the all-ones mask if (x, y) is on the curve; for an
 // off-curve y the reference goes on with x = sqrt(-1)*beta (garbage) — callers apply the SURVEY Q5
-// policy.  If negate is set the result is -P (x and t negated), which is what verify needs.
+// policy.  If negate is set the result is -P (x and t negated), which is what verify needs.  PUB: the public-data
+// flavour of the field operations (fe.cuh), for encodings that are public (verification, public-key conversion).
 //                                                                                 [ed_import, ed.c:100-149]
-EDG_HD u32 ge_frombytes(ge_p3 &p, const u32 in[8], bool negate, u32 *canonical = 0) {
+template <bool PUB = false> EDG_HD u32 ge_frombytes(ge_p3 &p, const u32 in[8], bool negate, u32 *canonical = 0) {
     const fe d = EDG_FE_D, sqrtm1 = EDG_FE_SQRTM1;
     u32 w[8];
 #pragma unroll
@@ -279,25 +273,25 @@ EDG_HD u32 ge_frombytes(ge_p3 &p, const u32 in[8], bool negate, u32 *canonical =
     fe one, yy, u, v, v3, v7, beta, chk, x, t;
     fe_set_u32(one, 1);
     fe_from_words(p.Y, w);
-    fe_sq(yy, p.Y);
-    fe_mul(v, yy, d);
-    fe_sub(u, yy, one);                                  // u = y^2 - 1
-    fe_add(v, v, one);                                   // v = d y^2 + 1
-    fe_sq(v3, v);
-    fe_mul(v3, v3, v);                                   // v^3
-    fe_sq(v7, v3);
-    fe_mul(v7, v7, v);                                   // v^7
-    fe_mul(t, u, v7);
-    fe_pow2523(t, t);                                    // (u v^7)^((p-5)/8)
-    fe_mul(t, t, v3);
-    fe_mul(beta, u, t);                                  // beta = u v^3 (u v^7)^((p-5)/8)    ed.c:121-131
-    fe_sq(chk, beta);
-    fe_mul(chk, chk, v);                                 // v beta^2
-    fe_sub(t, chk, u);
+    fe_sq_s<PUB>(yy, p.Y);
+    fe_mul_s<PUB>(v, yy, d);
+    fe_sub_s<PUB>(u, yy, one);                           // u = y^2 - 1
+    fe_add_s<PUB>(v, v, one);                            // v = d y^2 + 1
+    fe_sq_s<PUB>(v3, v);
+    fe_mul_s<PUB>(v3, v3, v);                            // v^3
+    fe_sq_s<PUB>(v7, v3);
+    fe_mul_s<PUB>(v7, v7, v);                            // v^7
+    fe_mul_s<PUB>(t, u, v7);
+    fe_pow_chain<PUB>(&t, &t, 0);                        // (u v^7)^((p-5)/8)
+    fe_mul_s<PUB>(t, t, v3);
+    fe_mul_s<PUB>(beta, u, t);                           // beta = u v^3 (u v^7)^((p-5)/8)    ed.c:121-131
+    fe_sq_s<PUB>(chk, beta);
+    fe_mul_s<PUB>(chk, chk, v);                          // v beta^2
+    fe_sub_s<PUB>(t, chk, u);
     const u32 is_root = 0u - fe_is_zero(t);              // v beta^2 == u                      ed.c:134-137
-    fe_add(t, chk, u);
+    fe_add_s<PUB>(t, chk, u);
     const u32 is_jroot = 0u - fe_is_zero(t);             // v beta^2 == -u  <=>  v (j beta)^2 == u
-    fe_mul(t, beta, sqrtm1);
+    fe_mul_s<PUB>(t, beta, sqrtm1);
     fe_select(x, t, beta, is_root);                      // x = is_root ? beta : j beta        ed.c:140-142
     fe_canon(x, x);
     if (canonical) {
@@ -312,9 +306,9 @@ EDG_HD u32 ge_frombytes(ge_p3 &p, const u32 in[8], bool negate, u32 *canonical =
     }
     u32 flip = 0u - ((sign ^ (x.v[0] & 1u)) & 1u);       // ed.c:143-144
     if (negate) flip = ~flip;
-    fe_neg(t, x);                                        // -0 stays == 0 mod p
+    fe_neg_s<PUB>(t, x);                                 // -0 stays == 0 mod p
     fe_select(p.X, x, t, flip);
-    fe_mul(p.T, p.X, p.Y);
+    fe_mul_s<PUB>(p.T, p.X, p.Y);
     fe_set_u32(p.Z, 1);
     return is_root | is_jroot;
 }

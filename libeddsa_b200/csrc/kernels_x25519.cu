@@ -64,6 +64,13 @@ __global__ void __launch_bounds__(kThreads) k_fe_selftest(size_t n, uint8_t *out
         case 6: fe_inv(r, x); break;
         case 7: fe_pow2523(r, x); break;
         case 8: fe_neg(r, x); break;
+        // 10..15: the public-data flavour of ops 0, 1, 2, 3, 8, 7, pending carries settled (bit-identical to those ops)
+        case 10: { const bool p = pub_mul(r, x, y); pub_settle_add(r, p); break; }
+        case 11: { const bool p = pub_sq(r, x); pub_settle_add(r, p); break; }
+        case 12: { const bool p = pub_add(r, x, y); pub_settle_add(r, p); break; }
+        case 13: { const bool p = pub_sub(r, x, y); pub_settle_sub(r, p); break; }
+        case 14: { const bool p = pub_neg(r, x); pub_settle_sub(r, p); break; }
+        case 15: pub_pow2523(r, x); break;
         default: fe_copy(r, x); break;
         }
         store8(out, i, r.v);

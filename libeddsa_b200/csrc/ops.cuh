@@ -417,17 +417,18 @@ EDG_HD void load_words8(u32 w[8], const u32 *src) {
 static int edg_last_nwin = 0;                              // host-only instrumentation (tests/host_sim): windows of the last verify
 #endif
 
-// Table k*Q, k = 0..8, in cached form, 9 x 32 words of this thread's scratch.       [ed_precompute, ed.c:436]
+// Table k*Q, k = 0..8, in cached form, 9 x 32 words of this thread's scratch (Q public: pub_ field operations).
+//                                                                                  [ed_precompute, ed.c:436]
 EDG_HD void ge_cached_table(u32 *tab, ge_p3 &Q) {
     ge_cached c, c1;
     fe_set_u32(c.ypx, 1); fe_set_u32(c.ymx, 1); fe_set_u32(c.z2, 2); fe_set_u32(c.t2d, 0);
     ge_cached_store(tab, c);
-    ge_to_cached(c1, Q);
+    ge_to_cached<true>(c1, Q);
     ge_cached_store(tab + 32, c1);
 #pragma unroll 1
     for (int k = 2; k <= 8; k++) {
-        ge_add_cached(Q, Q, c1, true);                    // k*Q = (k-1)*Q + Q
-        ge_to_cached(c, Q);
+        ge_add_cached<true>(Q, Q, c1, true);              // k*Q = (k-1)*Q + Q
+        ge_to_cached<true>(c, Q);
         ge_cached_store(tab + 32 * k, c);
     }
 }
@@ -500,7 +501,7 @@ EDG_HD void ed25519_verify_front_points(u32 *state, const u32 *sig, const u32 *p
         ge_p3 Q;
         u32 a[8], canon;
         load_words8(a, which ? sig : pub);
-        good &= ge_frombytes(Q, a, true, &canon);
+        good &= ge_frombytes<true>(Q, a, true, &canon);
         good &= which ? canon : 0xffffffffu;              // only R has to be canonical (Q2); any encoding of A is accepted (Q3)
         ge_cached_table(state + 288 * which, Q);
     }
@@ -561,19 +562,25 @@ EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0
 #endif
 #pragma unroll 1
         for (int step = (j == nwin - 1 ? 4 : 0); step < last; step++) {
+            // Public data only: the field operations are the pub_ flavour (fe.cuh), in groups of independent operations
+            // whose pending carries are settled by one rarely taken branch per group.
             fe e, f, g, h;
+            bool p0, p1, p2, p3;
             if (step < 4) {                                   // doubling prologue                 [ed_double, ed.c:211]
                 fe a, b, c, s;
-                fe_sq(a, R.X);
-                fe_sq(b, R.Y);
-                fe_sq(c, R.Z);
-                fe_dbl(c, c);
-                fe_add(s, R.X, R.Y);
-                fe_sq(s, s);
-                fe_add(h, a, b);
-                fe_sub(e, h, s);
-                fe_sub(g, a, b);
-                fe_add(f, c, g);
+                p0 = pub_sq(a, R.X);
+                p1 = pub_sq(b, R.Y);
+                p2 = pub_sq(c, R.Z);
+                p3 = pub_add(s, R.X, R.Y);
+                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(a, p0); pub_settle_add(b, p1); pub_settle_add(c, p2); pub_settle_add(s, p3); }
+                p0 = pub_dbl(c, c);
+                p1 = pub_sq(s, s);
+                p2 = pub_add(h, a, b);
+                p3 = pub_sub(g, a, b);
+                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(c, p0); pub_settle_add(s, p1); pub_settle_add(h, p2); pub_settle_sub(g, p3); }
+                p0 = pub_sub(e, h, s);
+                p1 = pub_add(f, c, g);
+                if (pub_rare(p0 | p1)) { pub_settle_sub(e, p0); pub_settle_add(f, p1); }
             } else {                                          // addition prologue                 [ed_add ed.c:175 / ed_add_pc :282]
                 fe ypx, ymx, t2d, a, b, c, d;
                 if (step < 6) {                               // digit * Q or digit * P: cached entry from this thread's scratch
@@ -594,31 +601,42 @@ EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0
                     } else
 #endif
                     ge_cached_load(q, qtab + (step == 4 ? 0 : 288) + 32 * absd);
-                    ge_cached_cneg(q, neg);
-                    fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx); fe_copy(t2d, q.t2d);
-                    fe_mul(d, R.Z, q.z2);
+                    fe nt;                                    // q = neg ? -q : q  (ge_cached_cneg, negation in the group below)
+                    fe_cswap(q.ypx, q.ymx, neg);
+                    fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx);
+                    p0 = pub_neg(nt, q.t2d);
+                    p1 = pub_mul(d, R.Z, q.z2);
+                    p2 = pub_sub(a, R.Y, R.X);
+                    p3 = pub_add(b, R.Y, R.X);
+                    if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_sub(nt, p0); pub_settle_add(d, p1); pub_settle_sub(a, p2); pub_settle_add(b, p3); }
+                    fe_select(t2d, q.t2d, nt, neg);
                 } else {                                      // digit * B or digit * 2^128 B: affine entry of a window table (Z2 = 1)
                     const int k = (j >> 2) + (step == 6 ? 0 : 8);
                     const int ds = (int)((es[k >> 1] >> (16 * (k & 1))) & 0xffffu) - 0x8000;
                     ge_pre q;
                     ge_pre_load_wtab(q, wtab + (step == 6 ? 0u : EDG_WTAB_WORDS), ds);
                     fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx); fe_copy(t2d, q.xy2d);
-                    fe_dbl(d, R.Z);
+                    p0 = pub_dbl(d, R.Z);
+                    p2 = pub_sub(a, R.Y, R.X);
+                    p3 = pub_add(b, R.Y, R.X);
+                    if (pub_rare(p0 | p2 | p3)) { pub_settle_add(d, p0); pub_settle_sub(a, p2); pub_settle_add(b, p3); }
                 }
-                fe_sub(a, R.Y, R.X);
-                fe_mul(a, a, ymx);
-                fe_add(b, R.Y, R.X);
-                fe_mul(b, b, ypx);
-                fe_mul(c, R.T, t2d);
-                fe_sub(e, b, a);
-                fe_sub(f, d, c);
-                fe_add(g, d, c);
-                fe_add(h, b, a);
+                p0 = pub_mul(a, a, ymx);
+                p1 = pub_mul(b, b, ypx);
+                p2 = pub_mul(c, R.T, t2d);
+                if (pub_rare(p0 | p1 | p2)) { pub_settle_add(a, p0); pub_settle_add(b, p1); pub_settle_add(c, p2); }
+                p0 = pub_sub(e, b, a);
+                p1 = pub_sub(f, d, c);
+                p2 = pub_add(g, d, c);
+                p3 = pub_add(h, b, a);
+                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_sub(e, p0); pub_settle_sub(f, p1); pub_settle_add(g, p2); pub_settle_add(h, p3); }
             }
-            fe_mul(R.X, e, f);                                // shared tail
-            fe_mul(R.Y, g, h);
-            fe_mul(R.Z, f, g);
-            if (step == 3 || step == 4 || step == 6 || (step == 5 && has_b)) fe_mul(R.T, e, h);
+            p0 = pub_mul(R.X, e, f);                          // shared tail
+            p1 = pub_mul(R.Y, g, h);
+            p2 = pub_mul(R.Z, f, g);
+            p3 = false;
+            if (step == 3 || step == 4 || step == 6 || (step == 5 && has_b)) p3 = pub_mul(R.T, e, h);
+            if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(R.X, p0); pub_settle_add(R.Y, p1); pub_settle_add(R.Z, p2); pub_settle_add(R.T, p3); }
         }
     }
     // the sum is the neutral element (0 : 1 : 1)  <=>  X = 0 and Y = Z   (Z != 0: the addition law is complete)

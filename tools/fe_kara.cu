@@ -70,7 +70,7 @@ __device__ __forceinline__ void fe_mul_k(fe &r, const fe &a, const fe &b) {
         "addc.cc.u32 %10, %10, 0; addc.u32 %11, %11, 0;"
         : "+r"(w[4]), "+r"(w[5]), "+r"(w[6]), "+r"(w[7]), "+r"(w[8]), "+r"(w[9]), "+r"(w[10]), "+r"(w[11]), "+r"(w[12]), "+r"(w[13]), "+r"(w[14]), "+r"(w[15])
         : "r"(mid[0]), "r"(mid[1]), "r"(mid[2]), "r"(mid[3]), "r"(mid[4]), "r"(mid[5]), "r"(mid[6]), "r"(mid[7]), "r"(mid[8]));
-    fe_fold_sq(r, w);
+    fe_fold_sq<false>(r, w);
 #endif
 }
 
@@ -106,7 +106,7 @@ __device__ __forceinline__ void fe_sq_v(fe &r, const fe &a) {
           "+r"(w[12]), "+r"(w[13]), "+r"(w[14]), "+r"(w[15])
         : "r"(d[0]), "r"(d[1]), "r"(d[2]), "r"(d[3]), "r"(d[4]), "r"(d[5]), "r"(d[6]), "r"(d[7]), "r"(d[8]), "r"(d[9]), "r"(d[10]), "r"(d[11]),
           "r"(d[12]), "r"(d[13]), "r"(d[14]), "r"(d[15]));
-    fe_fold_sq(r, w);
+    fe_fold_sq<false>(r, w);
 #endif
 }
 
