@@ -52,6 +52,20 @@ EDDSA_DECL int ed25519_sign_batch(size_t n, uint8_t *sig, const uint8_t *sec, co
 /* batch of ed25519_verify (reference eddsa.h:52, ed25519-sha512.c:148) */
 EDDSA_DECL int ed25519_verify_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
                                     const uint8_t *msgs, const size_t *off, size_t fixed_len);
+/* Batch verification under a chosen acceptance rule.  t = SHA-512(R || A || M) mod L over the bytes as given, always.
+ *                      S            A encoding          R encoding          small-order A, R   equation
+ *   REFERENCE (0)      mod L        any (y >= p, "-0")  canonical           allowed            S B - t A - R == O
+ *   STRICT    (1)      S < L        canonical           canonical           rejected           S B - t A - R == O
+ *   ZIP215    (2)      S < L        any                 any (decoded as A)  allowed            8 (S B - t A - R) == O
+ * Off-curve A or R are rejected by every rule.  REFERENCE is ed25519_verify_batch (libeddsa v0.8); STRICT is RFC 8032
+ * with canonical encodings and what libsodium's crypto_sign_verify_detached decides (non-malleable); ZIP215 is Zcash's
+ * ZIP 215 (consensus: every encoding of a point, cofactored).  Layouts and behaviour are those of ed25519_verify_batch
+ * / ed25519_verify_batch_dev; an unknown policy returns EDDSA_B200_EINVAL before any work, even when n = 0. */
+#define EDDSA_B200_VERIFY_REFERENCE 0   /* = ed25519_verify_batch */
+#define EDDSA_B200_VERIFY_STRICT    1   /* RFC 8032 with canonical encodings, no small-order A or R (libsodium) */
+#define EDDSA_B200_VERIFY_ZIP215    2   /* ZIP 215: any encoding, S < L, cofactored */
+EDDSA_DECL int ed25519_verify_policy_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
+                                           const uint8_t *msgs, const size_t *off, size_t fixed_len, int policy);
 /* batch of x25519 (reference eddsa.h:67, x25519.c:215) */
 EDDSA_DECL int x25519_batch(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point);
 /* batch of x25519_base (reference eddsa.h:64, x25519.c:203) */
@@ -66,6 +80,9 @@ EDDSA_DECL int ed25519_sign_batch_dev(size_t n, uint8_t *sig, const uint8_t *sec
                                       const uint8_t *msgs, const uint64_t *off, size_t fixed_len, void *stream);
 EDDSA_DECL int ed25519_verify_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
                                         const uint8_t *msgs, const uint64_t *off, size_t fixed_len, void *stream);
+EDDSA_DECL int ed25519_verify_policy_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
+                                               const uint8_t *msgs, const uint64_t *off, size_t fixed_len,
+                                               int policy, void *stream);
 EDDSA_DECL int x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point, void *stream);
 EDDSA_DECL int x25519_base_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, void *stream);
 EDDSA_DECL int pk_ed25519_to_x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *in, void *stream);

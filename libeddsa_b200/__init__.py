@@ -25,6 +25,11 @@ ED25519_KEY_LEN = 32
 ED25519_SIG_LEN = 64
 X25519_KEY_LEN = 32
 
+# acceptance rules of ed25519_verify_policy_batch / _dev (include/eddsa_batch.h: EDDSA_B200_VERIFY_*)
+VERIFY_REFERENCE = 0   # libeddsa v0.8, what ed25519_verify_batch decides: S mod L, any A encoding, cofactorless
+VERIFY_STRICT = 1      # RFC 8032 with canonical encodings (libsodium): S < L, canonical A and R, no small-order A or R
+VERIFY_ZIP215 = 2      # ZIP 215: S < L, any encoding of A and R, cofactored
+
 
 class EddsaB200Error(RuntimeError):
     pass
@@ -53,6 +58,7 @@ def lib():
             "ed25519_genpub_batch": [sz, vp, vp],
             "ed25519_sign_batch": [sz, vp, vp, vp, vp, vp, sz],
             "ed25519_verify_batch": [sz, vp, vp, vp, vp, vp, sz],
+            "ed25519_verify_policy_batch": [sz, vp, vp, vp, vp, vp, sz, ip],
             "x25519_batch": [sz, vp, vp, vp],
             "x25519_base_batch": [sz, vp, vp],
             "pk_ed25519_to_x25519_batch": [sz, vp, vp],
@@ -60,6 +66,7 @@ def lib():
             "ed25519_genpub_batch_dev": [sz, vp, vp, vp],
             "ed25519_sign_batch_dev": [sz, vp, vp, vp, vp, vp, sz, vp],
             "ed25519_verify_batch_dev": [sz, vp, vp, vp, vp, vp, sz, vp],
+            "ed25519_verify_policy_batch_dev": [sz, vp, vp, vp, vp, vp, sz, ip, vp],
             "x25519_batch_dev": [sz, vp, vp, vp, vp],
             "x25519_base_batch_dev": [sz, vp, vp, vp],
             "pk_ed25519_to_x25519_batch_dev": [sz, vp, vp, vp],
@@ -168,6 +175,18 @@ def ed25519_verify_batch(sig, pub, msgs, off=None, fixed_len=0):
     msgs, off = _msgs(msgs, off, fixed_len, len(sig))
     ok = np.empty(len(sig), np.uint8)
     _check(lib().ed25519_verify_batch(len(sig), _p(ok), _p(sig), _p(pub), _p(msgs), _p(off), fixed_len), "ed25519_verify_batch")
+    return ok
+
+
+def ed25519_verify_policy_batch(sig, pub, msgs, off=None, fixed_len=0, policy=VERIFY_STRICT):
+    """ed25519_verify_batch under the acceptance rule `policy` (VERIFY_REFERENCE, VERIFY_STRICT or VERIFY_ZIP215)."""
+    sig, pub = _arr(sig, 64, "sig"), _arr(pub, 32, "pub")
+    if len(sig) != len(pub):
+        raise ValueError("sig / pub length mismatch")
+    msgs, off = _msgs(msgs, off, fixed_len, len(sig))
+    ok = np.empty(len(sig), np.uint8)
+    _check(lib().ed25519_verify_policy_batch(len(sig), _p(ok), _p(sig), _p(pub), _p(msgs), _p(off), fixed_len, policy),
+           "ed25519_verify_policy_batch")
     return ok
 
 
@@ -322,6 +341,12 @@ def ed25519_sign_batch_dev(sig, sec, pub, msgs, off=None, fixed_len=0):
 def ed25519_verify_batch_dev(ok, sig, pub, msgs, off=None, fixed_len=0):
     n = sig.numel() // 64
     _check(lib().ed25519_verify_batch_dev(n, _dp(ok), _dp(sig), _dp(pub), _dp(msgs), _dp(off), fixed_len, _stream()), "ed25519_verify_batch_dev")
+
+
+def ed25519_verify_policy_batch_dev(ok, sig, pub, msgs, off=None, fixed_len=0, policy=VERIFY_STRICT):
+    n = sig.numel() // 64
+    _check(lib().ed25519_verify_policy_batch_dev(n, _dp(ok), _dp(sig), _dp(pub), _dp(msgs), _dp(off), fixed_len, policy, _stream()),
+           "ed25519_verify_policy_batch_dev")
 
 
 def x25519_batch_dev(out, scalar, point):

@@ -41,6 +41,10 @@ void edg_verify_debug_full_scalars(int on);      /* test hook: force the full-le
 int edg_launch_verify(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                       const unsigned long long *off, unsigned long long fixed_len, void *scratch, size_t records, const void *table,
                       int sm_count, void *stream, unsigned *launches);
+/* the same under the acceptance rule `policy` (EDDSA_B200_VERIFY_* of eddsa_batch.h); policy 0 is edg_launch_verify */
+int edg_launch_verify_policy(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                             const unsigned long long *off, unsigned long long fixed_len, int policy, void *scratch, size_t records,
+                             const void *table, int sm_count, void *stream, unsigned *launches);
 
 int edg_launch_pk_convert(size_t n, uint8_t *out, const uint8_t *in, int sm_count, void *stream);
 int edg_launch_sk_convert(size_t n, uint8_t *out, const uint8_t *in, int sm_count, void *stream);

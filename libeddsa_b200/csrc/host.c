@@ -30,6 +30,11 @@
 #include "eddsa_batch.h"
 #include "edg_internal.h"
 
+/* Weak: the host layer also links against sets of launchers that only implement the reference's verify rule (the mock kernels
+ * of the test suite's CUDA runtime simulator).  There the address is NULL and the other rules are refused (bad_policy);
+ * kernels_verify.cu always defines it. */
+#pragma weak edg_launch_verify_policy
+
 #define EDG_MAX_DEV 16
 #define EDG_NSLOT 3
 #define EDG_ALIGN 256
@@ -53,6 +58,7 @@ typedef struct {
     size_t fixed_len;
     uint8_t *out;
     size_t out_item;
+    int policy;                                 /* verify: EDDSA_B200_VERIFY_* */
 } edg_job_t;
 
 struct shard;
@@ -293,7 +299,7 @@ static int is_pinned(const void *p)
 /* Enqueue one operation on `stream` (device of c current).  Kernel scratch comes from the context's stream-ordered
  * pool: allocated and freed on the same stream, so back-to-back calls reuse it without synchronising. */
 static int launch(edg_dev_t *c, edg_op_t op, size_t n, uint8_t *d_out, uint8_t *const d_in[3], const uint8_t *d_msgs,
-                  const unsigned long long *d_off, size_t fixed_len, void *stream)
+                  const unsigned long long *d_off, size_t fixed_len, int policy, void *stream)
 {
     int rc = 0;
     void *scratch = NULL;
@@ -306,7 +312,12 @@ static int launch(edg_dev_t *c, edg_op_t op, size_t n, uint8_t *d_out, uint8_t *
     switch (op) {
     case OP_GENPUB: rc = edg_launch_genpub(n, d_out, d_in[0], scratch, c->comb, c->sm_count, stream, &launches); break;
     case OP_SIGN: rc = edg_launch_sign(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, scratch, c->comb, c->sm_count, stream, &launches); break;
-    case OP_VERIFY: rc = edg_launch_verify(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, scratch, records, c->wtab, c->sm_count, stream, &launches); break;
+    case OP_VERIFY:
+        rc = policy == EDDSA_B200_VERIFY_REFERENCE
+                 ? edg_launch_verify(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, scratch, records, c->wtab, c->sm_count, stream, &launches)
+                 : edg_launch_verify_policy(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, policy, scratch, records, c->wtab, c->sm_count,
+                                            stream, &launches);
+        break;
     case OP_X25519: rc = edg_launch_x25519(n, d_out, d_in[0], d_in[1], c->sm_count, stream); launches = 1; break;
     case OP_X25519_BASE: rc = edg_launch_x25519_base(n, d_out, d_in[0], c->comb, c->sm_count, stream); launches = 1; break;
     case OP_PK_CONV: rc = edg_launch_pk_convert(n, d_out, d_in[0], c->sm_count, stream); launches = 1; break;
@@ -554,12 +565,12 @@ static int run_shard(edg_dev_t *c, const edg_job_t *j, size_t lo, size_t hi)
         if (j->op == OP_VERIFY) {
             CU(cudaEventRecord(c->in_ready[s], c->stream[s]));
             CU(cudaStreamWaitEvent(c->kstream, c->in_ready[s], 0));
-            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, c->kstream);
+            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, j->policy, c->kstream);
             if (rc) goto out;
             CU(cudaEventRecord(c->k_done[s], c->kstream));
             CU(cudaStreamWaitEvent(c->stream[s], c->k_done[s], 0));
         } else {
-            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, c->stream[s]);
+            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, j->policy, c->stream[s]);
             if (rc) goto out;
         }
         if (secret_in) CU(cudaMemsetAsync(c->d_in[s], 0, m * j->in_item[0], c->stream[s]));        /* the secret keys of this chunk */
@@ -707,45 +718,60 @@ static int run_job(const edg_job_t *j)
  * --------------------------------------------------------------------------------------------- */
 int ed25519_genpub_batch(size_t n, uint8_t *pub, const uint8_t *sec)
 {
-    edg_job_t j = {OP_GENPUB, n, 1, {sec, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, pub, 32};
+    edg_job_t j = {OP_GENPUB, n, 1, {sec, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, pub, 32, 0};
     return run_job(&j);
 }
 
 int ed25519_sign_batch(size_t n, uint8_t *sig, const uint8_t *sec, const uint8_t *pub, const uint8_t *msgs,
                        const size_t *off, size_t fixed_len)
 {
-    edg_job_t j = {OP_SIGN, n, 2, {sec, pub, NULL}, {32, 32, 0}, 1, msgs, off, fixed_len, sig, 64};
+    edg_job_t j = {OP_SIGN, n, 2, {sec, pub, NULL}, {32, 32, 0}, 1, msgs, off, fixed_len, sig, 64, 0};
     return run_job(&j);
+}
+
+static int bad_policy(int policy)
+{
+    t_err[0] = 0;
+    if (policy == EDDSA_B200_VERIFY_REFERENCE) return 0;
+    if (policy != EDDSA_B200_VERIFY_STRICT && policy != EDDSA_B200_VERIFY_ZIP215) return fail(EDDSA_B200_EINVAL, "unknown verify policy %d", policy);
+    if (!edg_launch_verify_policy) return fail(EDDSA_B200_EINVAL, "verify policy %d: these kernels have no launcher for it", policy);
+    return 0;
+}
+
+int ed25519_verify_policy_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                                const size_t *off, size_t fixed_len, int policy)
+{
+    edg_job_t j = {OP_VERIFY, n, 2, {sig, pub, NULL}, {64, 32, 0}, 1, msgs, off, fixed_len, ok, 1, policy};
+    return bad_policy(policy) ? EDDSA_B200_EINVAL : run_job(&j);
 }
 
 int ed25519_verify_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                          const size_t *off, size_t fixed_len)
 {
-    edg_job_t j = {OP_VERIFY, n, 2, {sig, pub, NULL}, {64, 32, 0}, 1, msgs, off, fixed_len, ok, 1};
-    return run_job(&j);
+    return ed25519_verify_policy_batch(n, ok, sig, pub, msgs, off, fixed_len, EDDSA_B200_VERIFY_REFERENCE);
 }
 
 int x25519_batch(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point)
 {
-    edg_job_t j = {OP_X25519, n, 2, {scalar, point, NULL}, {32, 32, 0}, 0, NULL, NULL, 0, out, 32};
+    edg_job_t j = {OP_X25519, n, 2, {scalar, point, NULL}, {32, 32, 0}, 0, NULL, NULL, 0, out, 32, 0};
     return run_job(&j);
 }
 
 int x25519_base_batch(size_t n, uint8_t *out, const uint8_t *scalar)
 {
-    edg_job_t j = {OP_X25519_BASE, n, 1, {scalar, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32};
+    edg_job_t j = {OP_X25519_BASE, n, 1, {scalar, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0};
     return run_job(&j);
 }
 
 int pk_ed25519_to_x25519_batch(size_t n, uint8_t *out, const uint8_t *in)
 {
-    edg_job_t j = {OP_PK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32};
+    edg_job_t j = {OP_PK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0};
     return run_job(&j);
 }
 
 int sk_ed25519_to_x25519_batch(size_t n, uint8_t *out, const uint8_t *in)
 {
-    edg_job_t j = {OP_SK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32};
+    edg_job_t j = {OP_SK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0};
     return run_job(&j);
 }
 
@@ -754,7 +780,7 @@ int sk_ed25519_to_x25519_batch(size_t n, uint8_t *out, const uint8_t *in)
  * items); a, b, out: n x 32 bytes, any 256-bit values */
 int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, int op)
 {
-    edg_job_t j = {OP_FE_TEST, n, 2, {a, b, NULL}, {32, 32, 0}, 0, NULL, NULL, (size_t)op, out, 32};
+    edg_job_t j = {OP_FE_TEST, n, 2, {a, b, NULL}, {32, 32, 0}, 0, NULL, NULL, (size_t)op, out, 32, 0};
     return run_job(&j);
 }
 
@@ -764,7 +790,7 @@ int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8
  * 2^(16 k), the signed 16-bit digits of a < 2^253 as the verify loop reads them); a, b, c, out: n x 32 bytes */
 int eddsa_b200_sc_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *c, int op)
 {
-    edg_job_t j = {OP_SC_TEST, n, 3, {a, b, c}, {32, 32, 32}, 0, NULL, NULL, (size_t)op, out, 32};
+    edg_job_t j = {OP_SC_TEST, n, 3, {a, b, c}, {32, 32, 32}, 0, NULL, NULL, (size_t)op, out, 32, 0};
     return run_job(&j);
 }
 
@@ -826,7 +852,7 @@ size_t eddsa_b200_debug_peek_staging(int which, int slot, uint8_t *out, size_t l
 static int misaligned(const void *p) { return ((uintptr_t)p & 15) != 0; }
 
 static int dev_call(edg_op_t op, size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *msgs,
-                    const uint64_t *off, size_t fixed_len, void *stream)
+                    const uint64_t *off, size_t fixed_len, int policy, void *stream)
 {
     edg_dev_t *c;
     uint8_t *d_in[3] = {(uint8_t *)a, (uint8_t *)b, NULL};
@@ -838,47 +864,54 @@ static int dev_call(edg_op_t op, size_t n, uint8_t *out, const uint8_t *a, const
         return fail(EDDSA_B200_EINVAL, "device arrays must be non-NULL and 16-byte aligned");
     if ((op == OP_SIGN || op == OP_VERIFY) && !msgs && (off || fixed_len))
         return fail(EDDSA_B200_EINVAL, "NULL message blob");
-    return launch(c, op, n, out, d_in, msgs, (const unsigned long long *)off, fixed_len, stream);
+    return launch(c, op, n, out, d_in, msgs, (const unsigned long long *)off, fixed_len, policy, stream);
 }
 
 int ed25519_genpub_batch_dev(size_t n, uint8_t *pub, const uint8_t *sec, void *stream)
 {
-    return dev_call(OP_GENPUB, n, pub, sec, NULL, NULL, NULL, 0, stream);
+    return dev_call(OP_GENPUB, n, pub, sec, NULL, NULL, NULL, 0, 0, stream);
 }
 
 int ed25519_sign_batch_dev(size_t n, uint8_t *sig, const uint8_t *sec, const uint8_t *pub, const uint8_t *msgs,
                            const uint64_t *off, size_t fixed_len, void *stream)
 {
     if (n && !pub) return fail(EDDSA_B200_EINVAL, "NULL pub array");
-    return dev_call(OP_SIGN, n, sig, sec, pub, msgs, off, fixed_len, stream);
+    return dev_call(OP_SIGN, n, sig, sec, pub, msgs, off, fixed_len, 0, stream);
+}
+
+int ed25519_verify_policy_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                                    const uint64_t *off, size_t fixed_len, int policy, void *stream)
+{
+    if (bad_policy(policy)) return EDDSA_B200_EINVAL;
+    if (n && !pub) return fail(EDDSA_B200_EINVAL, "NULL pub array");
+    return dev_call(OP_VERIFY, n, ok, sig, pub, msgs, off, fixed_len, policy, stream);
 }
 
 int ed25519_verify_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                              const uint64_t *off, size_t fixed_len, void *stream)
 {
-    if (n && !pub) return fail(EDDSA_B200_EINVAL, "NULL pub array");
-    return dev_call(OP_VERIFY, n, ok, sig, pub, msgs, off, fixed_len, stream);
+    return ed25519_verify_policy_batch_dev(n, ok, sig, pub, msgs, off, fixed_len, EDDSA_B200_VERIFY_REFERENCE, stream);
 }
 
 int x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point, void *stream)
 {
     if (n && !point) return fail(EDDSA_B200_EINVAL, "NULL point array");
-    return dev_call(OP_X25519, n, out, scalar, point, NULL, NULL, 0, stream);
+    return dev_call(OP_X25519, n, out, scalar, point, NULL, NULL, 0, 0, stream);
 }
 
 int x25519_base_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, void *stream)
 {
-    return dev_call(OP_X25519_BASE, n, out, scalar, NULL, NULL, NULL, 0, stream);
+    return dev_call(OP_X25519_BASE, n, out, scalar, NULL, NULL, NULL, 0, 0, stream);
 }
 
 int pk_ed25519_to_x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *in, void *stream)
 {
-    return dev_call(OP_PK_CONV, n, out, in, NULL, NULL, NULL, 0, stream);
+    return dev_call(OP_PK_CONV, n, out, in, NULL, NULL, NULL, 0, 0, stream);
 }
 
 int sk_ed25519_to_x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *in, void *stream)
 {
-    return dev_call(OP_SK_CONV, n, out, in, NULL, NULL, NULL, 0, stream);
+    return dev_call(OP_SK_CONV, n, out, in, NULL, NULL, NULL, 0, 0, stream);
 }
 
 /* ---------------------------------------------------------------------------------------------

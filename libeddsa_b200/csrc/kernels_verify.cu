@@ -94,20 +94,23 @@ __global__ void __launch_bounds__(kThreads, EDG_LB_VERIFY) k_verify_scalars(size
     }
 }
 
+// POLICY: the acceptance rule (ops.cuh: EDG_VERIFY_*); it decides the encoding rules in the flag word
+template <int POLICY>
 __global__ void __launch_bounds__(kThreads, EDG_LB_VERIFY) k_verify_points(size_t n, const uint8_t *sig, const uint8_t *pub, u32 *state) {
     const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < n) ed25519_verify_front_points(state + k * EDG_VSTATE_WORDS, reinterpret_cast<const u32 *>(sig + 64 * k), reinterpret_cast<const u32 *>(pub + 32 * k));
+    if (k < n) ed25519_verify_front_points<POLICY>(state + k * EDG_VSTATE_WORDS, reinterpret_cast<const u32 *>(sig + 64 * k), reinterpret_cast<const u32 *>(pub + 32 * k));
 }
 
 // the window loop.  Whole warps stay together (the trip count is agreed per warp with a full-mask reduction): lanes
-// past the end redo the last record and drop the result.
+// past the end redo the last record and drop the result.  COFACTORED: the ZIP215 rule.
+template <bool COFACTORED>
 __global__ void __launch_bounds__(kVThreads, EDG_LB_VLOOP) k_verify(size_t n, uint8_t *ok, const u32 *state, const unsigned int *perm,
                                                                    const u32 *__restrict__ wtab) {
     const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if ((j & ~(size_t)31) >= n) return;
     const unsigned k = perm[j < n ? j : n - 1];
     __shared__ uint4 s_stage[16 * kVThreads];                  // 2 table entries x 8 x 16 bytes per thread, chunk-major
-    const u32 r = ed25519_verify_loop(state + (size_t)k * EDG_VSTATE_WORDS, wtab, reinterpret_cast<u32 *>(s_stage));
+    const u32 r = ed25519_verify_loop<COFACTORED>(state + (size_t)k * EDG_VSTATE_WORDS, wtab, reinterpret_cast<u32 *>(s_stage));
     if (j < n) ok[k] = (uint8_t)r;
 }
 
@@ -143,7 +146,7 @@ extern "C" {
 // signatures per full pass: a whole number of waves of the loop kernel (resident threads of the device)
 size_t edg_verify_pass(int sm_count) {
     int bps = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_verify, kVThreads, 0) != cudaSuccess || bps < 1) bps = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_verify<false>, kVThreads, 0) != cudaSuccess || bps < 1) bps = 1;
     return (size_t)sm_count * bps * kVThreads * g_waves;
 }
 
@@ -172,11 +175,15 @@ int edg_verify_table_init(void *table, void *stream) {
 // test hook (EDDSA_B200_DEBUG_FULL_SCALARS=1): every signature takes the full-length fallback (rho, tau) = (1, t)
 void edg_verify_debug_full_scalars(int on) { g_full_scalars = on; }
 
-// scratch: edg_verify_scratch_bytes(records) bytes; a pass handles up to `records` signatures
-int edg_launch_verify(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
-                      const unsigned long long *off, unsigned long long fixed_len, void *scratch, size_t records, const void *table,
-                      int sm_count, void *stream, unsigned *launches) {
+// scratch: edg_verify_scratch_bytes(records) bytes; a pass handles up to `records` signatures; policy: EDG_VERIFY_*
+int edg_launch_verify_policy(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                             const unsigned long long *off, unsigned long long fixed_len, int policy, void *scratch, size_t records,
+                             const void *table, int sm_count, void *stream, unsigned *launches) {
     cudaStream_t st = (cudaStream_t)stream;
+    void (*points)(size_t, const uint8_t *, const uint8_t *, u32 *) =
+        policy == EDG_VERIFY_STRICT ? k_verify_points<EDG_VERIFY_STRICT> : policy == EDG_VERIFY_ZIP215 ? k_verify_points<EDG_VERIFY_ZIP215>
+                                                                         : k_verify_points<EDG_VERIFY_REFERENCE>;
+    void (*loop)(size_t, uint8_t *, const u32 *, const unsigned int *, const u32 *) = policy == EDG_VERIFY_ZIP215 ? k_verify<true> : k_verify<false>;
     u32 *state = (u32 *)scratch;
     unsigned int *perm = (unsigned int *)((uint8_t *)scratch + perm_offset(records));
     unsigned int *counters = (unsigned int *)((uint8_t *)scratch + counters_offset(records));
@@ -191,16 +198,23 @@ int edg_launch_verify(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *
             grid_for(k_verify_scalars<true>, m, 0, sm_count, &bps);
             const size_t tiles = (m + kMsgTile - 1) / kMsgTile, cap = (size_t)sm_count * bps;
             k_verify_scalars<true><<<(unsigned)(tiles < cap ? tiles : cap), kThreads, 0, st>>>(m, sg, pk, msgs, off + first, fixed_len, state, perm, counters, g_full_scalars);
-            k_verify_points<<<nb, kThreads, 0, st>>>(m, sg, pk, state);
+            points<<<nb, kThreads, 0, st>>>(m, sg, pk, state);
             *launches += 3;
         } else {
             k_verify_scalars<false><<<nb, kThreads, 0, st>>>(m, sg, pk, msgs + first * fixed_len, nullptr, fixed_len, state, perm, counters, g_full_scalars);
-            k_verify_points<<<nb, kThreads, 0, st>>>(m, sg, pk, state);
+            points<<<nb, kThreads, 0, st>>>(m, sg, pk, state);
             *launches += 3;
         }
-        k_verify<<<(unsigned)((m + kVThreads - 1) / kVThreads), kVThreads, 0, st>>>(m, ok + first, state, perm, (const u32 *)table);
+        loop<<<(unsigned)((m + kVThreads - 1) / kVThreads), kVThreads, 0, st>>>(m, ok + first, state, perm, (const u32 *)table);
     }
     return (int)cudaGetLastError();
+}
+
+int edg_launch_verify(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                      const unsigned long long *off, unsigned long long fixed_len, void *scratch, size_t records, const void *table,
+                      int sm_count, void *stream, unsigned *launches) {
+    return edg_launch_verify_policy(n, ok, sig, pub, msgs, off, fixed_len, EDG_VERIFY_REFERENCE, scratch, records, table, sm_count, stream,
+                                    launches);
 }
 
 int edg_launch_pk_convert(size_t n, uint8_t *out, const uint8_t *in, int sm_count, void *stream) {

@@ -418,7 +418,7 @@ static int edg_last_nwin = 0;                              // host-only instrume
 #endif
 
 // Table k*Q, k = 0..8, in cached form, 9 x 32 words of this thread's scratch (Q public: pub_ field operations).
-//                                                                                  [ed_precompute, ed.c:436]
+// Q is left holding 8*Q (the STRICT rule's small-order test reads it).             [ed_precompute, ed.c:436]
 EDG_HD void ge_cached_table(u32 *tab, ge_p3 &Q) {
     ge_cached c, c1;
     fe_set_u32(c.ypx, 1); fe_set_u32(c.ymx, 1); fe_set_u32(c.z2, 2); fe_set_u32(c.t2d, 0);
@@ -450,7 +450,8 @@ EDG_HD int sc_digit16(const u32 *e, int j) { return (int)((e[j >> 3] >> (4 * (j 
 //   loop : the window loop and the projective comparison with the neutral element
 // record: [0, 288) table of Q = -A, [288, 576) table of P = -R' (9 cached points x 32 words each),
 //         [576, 584) tau, [584, 592) |rho|, [592, 600) rho S recoded to signed 16-bit digits, [600] flags
-//         (bit 0: both points decoded and the R bytes are canonical), [601] windows needed, [602] sign of rho
+//         (bit 0: both points decoded and the encodings, S and the orders pass the acceptance rule — REFERENCE: the R bytes
+//         are canonical), [601] windows needed, [602] sign of rho
 //         (all-ones: the digits of tau are negated in the loop, i.e. Q stands for +A).
 // The scalar words [576, 600) + [601, 603) and the point words [0, 576) + [600] are written by two independent
 // stages (neither reads what the other writes), so they can run side by side; record k belongs to signature k of
@@ -493,32 +494,57 @@ EDG_HD void ed25519_verify_store_scalars(u32 *state, const verify_scalars &v, in
     state[602] = v.rho_neg ? 0xffffffffu : 0u;
 }
 
+// Acceptance rules (include/eddsa_batch.h: EDDSA_B200_VERIFY_*).  Everything a rule decides beyond the reference's
+// is a flag of the points stage or the cofactor of the loop; the scalars stage is the same for all three.
+//   0 REFERENCE  libeddsa: S reduced mod L, any encoding of A, canonical R, cofactorless
+//   1 STRICT     RFC 8032 with canonical encodings, as libsodium: S < L, canonical A and R, neither of small order
+//   2 ZIP215     ZIP 215: S < L, any encoding of A and R, cofactored (8 (S B - t A - R) == O)
+#define EDG_VERIFY_REFERENCE 0
+#define EDG_VERIFY_STRICT 1
+#define EDG_VERIFY_ZIP215 2
+
 // front, points: the tables of Q = -A and P = -R', flags.                                          :151, :174-175
+template <int POLICY = EDG_VERIFY_REFERENCE>
 EDG_HD void ed25519_verify_front_points(u32 *state, const u32 *sig, const u32 *pub) {
     u32 good = 0xffffffffu;
+    if constexpr (POLICY != EDG_VERIFY_REFERENCE) {      // S < L
+        u32 s[8];
+        load_words8(s, sig + 8);
+        good = 0u - sc_below_L(s);
+    }
 #pragma unroll 1
     for (int which = 0; which < 2; which++) {             // one loop body for both points: half the code
         ge_p3 Q;
         u32 a[8], canon;
         load_words8(a, which ? sig : pub);
         good &= ge_frombytes<true>(Q, a, true, &canon);
-        good &= which ? canon : 0xffffffffu;              // only R has to be canonical (Q2); any encoding of A is accepted (Q3)
+        if constexpr (POLICY == EDG_VERIFY_REFERENCE)
+            good &= which ? canon : 0xffffffffu;          // only R has to be canonical (Q2); any encoding of A is accepted (Q3)
+        else if constexpr (POLICY == EDG_VERIFY_STRICT)
+            good &= canon;
         ge_cached_table(state + 288 * which, Q);
+        if constexpr (POLICY == EDG_VERIFY_STRICT)      // Q now holds 8 (-A) / 8 (-R'): small order <=> it is the neutral element
+            good &= (fe_is_zero(Q.X) & fe_eq(Q.Y, Q.Z)) - 1u;
     }
     state[600] = good & 1u;
 }
 
+template <int POLICY = EDG_VERIFY_REFERENCE>
 EDG_HD void ed25519_verify_front(u32 *state, const u32 *sig, const u32 *pub, const uint8_t *msg, u64 len, bool full_scalars = false) {
     verify_scalars v;
     const int nwin = ed25519_verify_front_scalars(v, sig, pub, msg, len, full_scalars);
     ed25519_verify_store_scalars(state, v, nwin);
-    ed25519_verify_front_points(state, sig, pub);
+    ed25519_verify_front_points<POLICY>(state, sig, pub);
 }
 
 // stage (device only, may be null): this block's shared-memory staging area, 16 chunks x blockDim.x threads x 16 bytes.
 // At the start of a window every thread starts asynchronous copies (cp.async, no registers involved) of the two
 // table entries the window will add; they arrive while the four doublings run, so the additions find them in
 // shared memory instead of waiting ~1 us for the record in L2 / HBM (4.4 % of the loop's stall samples).
+// COFACTORED (ZIP215): three more doublings, as one extra pass j = -1 of the window loop that runs only the doubling
+// steps 0..2, before the comparison: 8 rho D == O.  That decides 8 D == O exactly: 8 D lies in the subgroup of prime
+// order L and 0 < |rho| < 2^128 < L (DESIGN.md §3.4).
+template <bool COFACTORED = false>
 EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0) {
     u32 et[8], er[8], es[8];
 #pragma unroll
@@ -544,11 +570,11 @@ EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0
     ge_p3 R;
     ge_identity(R);
 #pragma unroll 1
-    for (int j = nwin - 1; j >= 0; j--) {
+    for (int j = nwin - 1; j >= (COFACTORED ? -1 : 0); j--) {
         const bool has_b = ((j & 3) == 0) && j < 32;
-        const int last = has_b ? 8 : 6;
+        const int last = COFACTORED && j < 0 ? 3 : has_b ? 8 : 6;
 #if defined(__CUDA_ARCH__)
-        if (stage) {
+        if (stage && (!COFACTORED || j >= 0)) {
             const int d0 = sc_digit16(et, j), d1 = sc_digit16(er, j);
             const u32 *s0 = qtab + 32 * (d0 < 0 ? -d0 : d0), *s1 = qtab + 288 + 32 * (d1 < 0 ? -d1 : d1);
             const u32 dst = (u32)__cvta_generic_to_shared(stage) + 16u * threadIdx.x;
@@ -644,9 +670,13 @@ EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0
     return is_o & (good & 1u);
 }
 
-EDG_HD u32 ed25519_verify_op(const u32 *sig, const u32 *pub, const uint8_t *msg, u64 len, u32 *state, const u32 *wtab, bool full_scalars = false) {
-    ed25519_verify_front(state, sig, pub, msg, len, full_scalars);
-    return ed25519_verify_loop(state, wtab);
+EDG_HD u32 ed25519_verify_op(const u32 *sig, const u32 *pub, const uint8_t *msg, u64 len, u32 *state, const u32 *wtab, bool full_scalars = false,
+                             int policy = EDG_VERIFY_REFERENCE) {
+    switch (policy) {
+    case EDG_VERIFY_STRICT: ed25519_verify_front<EDG_VERIFY_STRICT>(state, sig, pub, msg, len, full_scalars); return ed25519_verify_loop<false>(state, wtab);
+    case EDG_VERIFY_ZIP215: ed25519_verify_front<EDG_VERIFY_ZIP215>(state, sig, pub, msg, len, full_scalars); return ed25519_verify_loop<true>(state, wtab);
+    default: ed25519_verify_front(state, sig, pub, msg, len, full_scalars); return ed25519_verify_loop(state, wtab);
+    }
 }
 
 // pk_ed25519_to_x25519: u = (1 + y) / (1 - y) of the decoded point.   [ed25519-sha512.c:187-237]

@@ -85,6 +85,15 @@ EDG_HD void sc_reduce512(u32 r[8], const u32 x[16]) {
     for (int i = 0; i < 8; i++) r[i] = v[i];
 }
 
+// 1 if the 256-bit value x is below L (a canonical scalar), else 0: the borrow out of x - L
+EDG_HD u32 sc_below_L(const u32 x[8]) {
+    const u32 Lw[9] = EDG_SC_L_INIT;
+    u32 borrow = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) borrow = (u32)(((u64)x[i] - Lw[i] - borrow) >> 63);
+    return borrow;
+}
+
 // 32-byte value (8 words, any value < 2^256) mod L.  No range check (SURVEY Q1).  [sc_import, sc.c:191]
 EDG_HD void sc_reduce256(u32 r[8], const u32 x[8]) {
     u32 w[16];
