@@ -66,6 +66,24 @@ EDDSA_DECL int ed25519_verify_batch(size_t n, uint8_t *ok, const uint8_t *sig, c
 #define EDDSA_B200_VERIFY_ZIP215    2   /* ZIP 215: any encoding, S < L, cofactored */
 EDDSA_DECL int ed25519_verify_policy_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
                                            const uint8_t *msgs, const size_t *off, size_t fixed_len, int policy);
+/* ZIP 215 decisions (EDDSA_B200_VERIFY_ZIP215), computed by randomised batch equations over groups of
+ * EDDSA_B200_VERIFY_BATCH_ROWS signatures, with an exact per-signature re-check of every group whose equation fails.
+ * Layouts, alignment, errors and streams are those of ed25519_verify_policy_batch[_dev].
+ *   - Every row ZIP 215 accepts is accepted.  A row ZIP 215 rejects is accepted with probability at most 2^-127 per group,
+ *     over the seed: the output equals ed25519_verify_policy_batch(..., EDDSA_B200_VERIFY_ZIP215).
+ *   - Row i's weight is z_i = SHA-512(seed || t_i || S_i)[0..16) with bit 0 set (t_i = SHA-512(R || A || M) mod L, 32
+ *     little-endian bytes), so it depends on the row's bytes only, not on its position.
+ *   - seed: 32 bytes (host memory, also for the _dev form), or NULL: 32 fresh bytes from getrandom(2), zeroed before the
+ *     call returns; if getrandom fails the call returns an error with nothing launched.  A caller-supplied seed makes the
+ *     output reproducible.  A seed known to signers makes the batch check worthless: they can craft invalid rows that
+ *     cancel.  Never reuse a seed across calls whose inputs an attacker chooses.
+ *   - Speed (one B200, 1000 W, 2^20 signatures of 64-byte messages): 1.16x per-signature ZIP 215 when all rows are valid,
+ *     1.13x with 0.1 % invalid rows, 0.63x when every group holds an invalid row (the batch pass plus a full per-signature
+ *     pass).  DESIGN.md §3.4 item 5. */
+#define EDDSA_B200_VERIFY_BATCH_ROWS 8          /* signatures per batch equation (one GPU thread) */
+EDDSA_DECL int ed25519_verify_zip215_batched(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
+                                             const uint8_t *msgs, const size_t *off, size_t fixed_len,
+                                             const uint8_t *seed);
 /* batch of x25519 (reference eddsa.h:67, x25519.c:215) */
 EDDSA_DECL int x25519_batch(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point);
 /* batch of x25519_base (reference eddsa.h:64, x25519.c:203) */
@@ -83,6 +101,9 @@ EDDSA_DECL int ed25519_verify_batch_dev(size_t n, uint8_t *ok, const uint8_t *si
 EDDSA_DECL int ed25519_verify_policy_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
                                                const uint8_t *msgs, const uint64_t *off, size_t fixed_len,
                                                int policy, void *stream);
+EDDSA_DECL int ed25519_verify_zip215_batched_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub,
+                                                 const uint8_t *msgs, const uint64_t *off, size_t fixed_len,
+                                                 const uint8_t *seed, void *stream);
 EDDSA_DECL int x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point, void *stream);
 EDDSA_DECL int x25519_base_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, void *stream);
 EDDSA_DECL int pk_ed25519_to_x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *in, void *stream);

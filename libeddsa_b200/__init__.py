@@ -29,6 +29,8 @@ X25519_KEY_LEN = 32
 VERIFY_REFERENCE = 0   # libeddsa v0.8, what ed25519_verify_batch decides: S mod L, any A encoding, cofactorless
 VERIFY_STRICT = 1      # RFC 8032 with canonical encodings (libsodium): S < L, canonical A and R, no small-order A or R
 VERIFY_ZIP215 = 2      # ZIP 215: S < L, any encoding of A and R, cofactored
+# signatures per batch equation of ed25519_verify_zip215_batched / _dev (include/eddsa_batch.h: EDDSA_B200_VERIFY_BATCH_ROWS)
+VERIFY_BATCH_ROWS = 8
 
 
 class EddsaB200Error(RuntimeError):
@@ -59,6 +61,7 @@ def lib():
             "ed25519_sign_batch": [sz, vp, vp, vp, vp, vp, sz],
             "ed25519_verify_batch": [sz, vp, vp, vp, vp, vp, sz],
             "ed25519_verify_policy_batch": [sz, vp, vp, vp, vp, vp, sz, ip],
+            "ed25519_verify_zip215_batched": [sz, vp, vp, vp, vp, vp, sz, vp],
             "x25519_batch": [sz, vp, vp, vp],
             "x25519_base_batch": [sz, vp, vp],
             "pk_ed25519_to_x25519_batch": [sz, vp, vp],
@@ -67,6 +70,7 @@ def lib():
             "ed25519_sign_batch_dev": [sz, vp, vp, vp, vp, vp, sz, vp],
             "ed25519_verify_batch_dev": [sz, vp, vp, vp, vp, vp, sz, vp],
             "ed25519_verify_policy_batch_dev": [sz, vp, vp, vp, vp, vp, sz, ip, vp],
+            "ed25519_verify_zip215_batched_dev": [sz, vp, vp, vp, vp, vp, sz, vp, vp],
             "x25519_batch_dev": [sz, vp, vp, vp, vp],
             "x25519_base_batch_dev": [sz, vp, vp, vp],
             "pk_ed25519_to_x25519_batch_dev": [sz, vp, vp, vp],
@@ -187,6 +191,28 @@ def ed25519_verify_policy_batch(sig, pub, msgs, off=None, fixed_len=0, policy=VE
     ok = np.empty(len(sig), np.uint8)
     _check(lib().ed25519_verify_policy_batch(len(sig), _p(ok), _p(sig), _p(pub), _p(msgs), _p(off), fixed_len, policy),
            "ed25519_verify_policy_batch")
+    return ok
+
+
+def _seed(seed):
+    if seed is None:
+        return None
+    seed = bytes(seed)
+    if len(seed) != 32:
+        raise ValueError("seed must be 32 bytes")
+    return ctypes.create_string_buffer(seed, 32)
+
+
+def ed25519_verify_zip215_batched(sig, pub, msgs, off=None, fixed_len=0, seed=None):
+    """ZIP 215 decisions (equal to ed25519_verify_policy_batch(..., VERIFY_ZIP215)) by randomised batch equations over
+    groups of VERIFY_BATCH_ROWS rows.  seed: 32 bytes, or None for fresh random bytes; never a value signers know."""
+    sig, pub = _arr(sig, 64, "sig"), _arr(pub, 32, "pub")
+    if len(sig) != len(pub):
+        raise ValueError("sig / pub length mismatch")
+    msgs, off = _msgs(msgs, off, fixed_len, len(sig))
+    ok = np.empty(len(sig), np.uint8)
+    _check(lib().ed25519_verify_zip215_batched(len(sig), _p(ok), _p(sig), _p(pub), _p(msgs), _p(off), fixed_len, _seed(seed)),
+           "ed25519_verify_zip215_batched")
     return ok
 
 
@@ -347,6 +373,12 @@ def ed25519_verify_policy_batch_dev(ok, sig, pub, msgs, off=None, fixed_len=0, p
     n = sig.numel() // 64
     _check(lib().ed25519_verify_policy_batch_dev(n, _dp(ok), _dp(sig), _dp(pub), _dp(msgs), _dp(off), fixed_len, policy, _stream()),
            "ed25519_verify_policy_batch_dev")
+
+
+def ed25519_verify_zip215_batched_dev(ok, sig, pub, msgs, off=None, fixed_len=0, seed=None):
+    n = sig.numel() // 64
+    _check(lib().ed25519_verify_zip215_batched_dev(n, _dp(ok), _dp(sig), _dp(pub), _dp(msgs), _dp(off), fixed_len, _seed(seed), _stream()),
+           "ed25519_verify_zip215_batched_dev")
 
 
 def x25519_batch_dev(out, scalar, point):

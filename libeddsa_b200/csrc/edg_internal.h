@@ -45,6 +45,13 @@ int edg_launch_verify(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *
 int edg_launch_verify_policy(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                              const unsigned long long *off, unsigned long long fixed_len, int policy, void *scratch, size_t records,
                              const void *table, int sm_count, void *stream, unsigned *launches);
+/* ZIP215 decisions by randomised batch equations over groups of EDG_VBATCH_K rows (ops.cuh), with the per-signature loop
+ * re-checking the rows of every failing equation; seed: 32 bytes in host memory (read before the call returns) */
+size_t edg_verify_batched_scratch_bytes(size_t records);
+void edg_verify_debug_no_fallback(int on);        /* test hook: failing equations write 0 and nothing is re-checked */
+int edg_launch_verify_batched(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                              const unsigned long long *off, unsigned long long fixed_len, const uint8_t *seed, void *scratch, size_t records,
+                              const void *table, int sm_count, void *stream, unsigned *launches);
 
 int edg_launch_pk_convert(size_t n, uint8_t *out, const uint8_t *in, int sm_count, void *stream);
 int edg_launch_sk_convert(size_t n, uint8_t *out, const uint8_t *in, int sm_count, void *stream);

@@ -19,11 +19,13 @@
  */
 #define _GNU_SOURCE
 #include <cuda_runtime_api.h>
+#include <errno.h>
 #include <pthread.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <sys/random.h>
 #include <unistd.h>
 
 #include "eddsa.h"
@@ -34,6 +36,10 @@
  * of the test suite's CUDA runtime simulator).  There the address is NULL and the other rules are refused (bad_policy);
  * kernels_verify.cu always defines it. */
 #pragma weak edg_launch_verify_policy
+/* The same for the batched ZIP215 check: where it is absent, its entry points are refused (batched_seed) */
+#pragma weak edg_launch_verify_batched
+#pragma weak edg_verify_batched_scratch_bytes
+#pragma weak edg_verify_debug_no_fallback
 
 #define EDG_MAX_DEV 16
 #define EDG_NSLOT 3
@@ -58,8 +64,12 @@ typedef struct {
     size_t fixed_len;
     uint8_t *out;
     size_t out_item;
-    int policy;                                 /* verify: EDDSA_B200_VERIFY_* */
+    int policy;                                 /* verify: EDDSA_B200_VERIFY_* or EDG_VERIFY_BATCHED */
+    const uint8_t *seed;                        /* EDG_VERIFY_BATCHED: the call's 32 seed bytes */
 } edg_job_t;
+
+/* internal verify policy: ZIP215 decided by batch equations (ed25519_verify_zip215_batched) */
+#define EDG_VERIFY_BATCHED 0x100
 
 struct shard;
 typedef struct {
@@ -150,6 +160,8 @@ static void global_init(void)
     __atomic_store_n(&g_nactive, g_nlist, __ATOMIC_RELEASE);
     if (env_int("EDDSA_B200_CHUNK_MB", 0) > 0) g_chunk_bytes = (size_t)env_int("EDDSA_B200_CHUNK_MB", 0) << 20;
     if (env_int("EDDSA_B200_DEBUG_FULL_SCALARS", 0) > 0) edg_verify_debug_full_scalars(1);
+    /* test hook: a failing batch equation writes 0 to its rows and nothing is re-checked (the raw equation) */
+    if (env_int("EDDSA_B200_DEBUG_NO_FALLBACK", 0) > 0 && edg_verify_debug_no_fallback) edg_verify_debug_no_fallback(1);
     if (env_int("EDDSA_B200_VERIFY_WAVES", 0) > 0) edg_verify_set_waves(env_int("EDDSA_B200_VERIFY_WAVES", 0));
     g_no_scrub = env_int("EDDSA_B200_DEBUG_NO_SCRUB", 0) > 0;   /* test hook: negative control of the staging-scrub test */
     /* helpers for big staging copies: a quarter of the host's cores per visible device, at most 3 — a host shared by one
@@ -299,20 +311,28 @@ static int is_pinned(const void *p)
 /* Enqueue one operation on `stream` (device of c current).  Kernel scratch comes from the context's stream-ordered
  * pool: allocated and freed on the same stream, so back-to-back calls reuse it without synchronising. */
 static int launch(edg_dev_t *c, edg_op_t op, size_t n, uint8_t *d_out, uint8_t *const d_in[3], const uint8_t *d_msgs,
-                  const unsigned long long *d_off, size_t fixed_len, int policy, void *stream)
+                  const unsigned long long *d_off, size_t fixed_len, int policy, const uint8_t *seed, void *stream)
 {
     int rc = 0;
     void *scratch = NULL;
     size_t need = 0, records = 0;
     unsigned launches = 0;
     if (n == 0) return 0;
-    if (op == OP_VERIFY) { records = n < c->verify_pass ? n : c->verify_pass; need = edg_verify_scratch_bytes(records); }   /* 2.4 KB per signature */
-    else if (op == OP_GENPUB || op == OP_SIGN) need = edg_fixedbase_scratch_bytes(op == OP_SIGN, n);
+    if (op == OP_VERIFY) {
+        records = n < c->verify_pass ? n : c->verify_pass;
+        need = policy == EDG_VERIFY_BATCHED ? edg_verify_batched_scratch_bytes(records)      /* + 96 B side record + 4 B per signature */
+                                            : edg_verify_scratch_bytes(records);              /* 2.4 KB per signature */
+    } else if (op == OP_GENPUB || op == OP_SIGN) need = edg_fixedbase_scratch_bytes(op == OP_SIGN, n);
     if (need) CU(cudaMallocFromPoolAsync(&scratch, need, c->pool, (cudaStream_t)stream));
     switch (op) {
     case OP_GENPUB: rc = edg_launch_genpub(n, d_out, d_in[0], scratch, c->comb, c->sm_count, stream, &launches); break;
     case OP_SIGN: rc = edg_launch_sign(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, scratch, c->comb, c->sm_count, stream, &launches); break;
     case OP_VERIFY:
+        if (policy == EDG_VERIFY_BATCHED) {
+            rc = edg_launch_verify_batched(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, seed, scratch, records, c->wtab, c->sm_count, stream,
+                                           &launches);
+            break;
+        }
         rc = policy == EDDSA_B200_VERIFY_REFERENCE
                  ? edg_launch_verify(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, scratch, records, c->wtab, c->sm_count, stream, &launches)
                  : edg_launch_verify_policy(n, d_out, d_in[0], d_in[1], d_msgs, d_off, fixed_len, policy, scratch, records, c->wtab, c->sm_count,
@@ -565,12 +585,12 @@ static int run_shard(edg_dev_t *c, const edg_job_t *j, size_t lo, size_t hi)
         if (j->op == OP_VERIFY) {
             CU(cudaEventRecord(c->in_ready[s], c->stream[s]));
             CU(cudaStreamWaitEvent(c->kstream, c->in_ready[s], 0));
-            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, j->policy, c->kstream);
+            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, j->policy, j->seed, c->kstream);
             if (rc) goto out;
             CU(cudaEventRecord(c->k_done[s], c->kstream));
             CU(cudaStreamWaitEvent(c->stream[s], c->k_done[s], 0));
         } else {
-            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, j->policy, c->stream[s]);
+            rc = launch(c, j->op, m, c->d_out[s], d_in, d_msgs, d_off, j->fixed_len, j->policy, j->seed, c->stream[s]);
             if (rc) goto out;
         }
         if (secret_in) CU(cudaMemsetAsync(c->d_in[s], 0, m * j->in_item[0], c->stream[s]));        /* the secret keys of this chunk */
@@ -718,14 +738,14 @@ static int run_job(const edg_job_t *j)
  * --------------------------------------------------------------------------------------------- */
 int ed25519_genpub_batch(size_t n, uint8_t *pub, const uint8_t *sec)
 {
-    edg_job_t j = {OP_GENPUB, n, 1, {sec, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, pub, 32, 0};
+    edg_job_t j = {OP_GENPUB, n, 1, {sec, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, pub, 32, 0, NULL};
     return run_job(&j);
 }
 
 int ed25519_sign_batch(size_t n, uint8_t *sig, const uint8_t *sec, const uint8_t *pub, const uint8_t *msgs,
                        const size_t *off, size_t fixed_len)
 {
-    edg_job_t j = {OP_SIGN, n, 2, {sec, pub, NULL}, {32, 32, 0}, 1, msgs, off, fixed_len, sig, 64, 0};
+    edg_job_t j = {OP_SIGN, n, 2, {sec, pub, NULL}, {32, 32, 0}, 1, msgs, off, fixed_len, sig, 64, 0, NULL};
     return run_job(&j);
 }
 
@@ -741,8 +761,34 @@ static int bad_policy(int policy)
 int ed25519_verify_policy_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                                 const size_t *off, size_t fixed_len, int policy)
 {
-    edg_job_t j = {OP_VERIFY, n, 2, {sig, pub, NULL}, {64, 32, 0}, 1, msgs, off, fixed_len, ok, 1, policy};
+    edg_job_t j = {OP_VERIFY, n, 2, {sig, pub, NULL}, {64, 32, 0}, 1, msgs, off, fixed_len, ok, 1, policy, NULL};
     return bad_policy(policy) ? EDDSA_B200_EINVAL : run_job(&j);
+}
+
+/* seed: the caller's 32 bytes, or (NULL) 32 fresh bytes from getrandom(2) in out, which the caller zeroes */
+static int batched_seed(uint8_t out[32], const uint8_t *seed)
+{
+    size_t got = 0;
+    t_err[0] = 0;
+    if (!edg_launch_verify_batched) return fail(EDDSA_B200_EINVAL, "batched ZIP215 verification: these kernels have no launcher for it");
+    if (seed) { memcpy(out, seed, 32); return 0; }
+    while (got < 32) {
+        ssize_t r = getrandom(out + got, 32 - got, 0);
+        if (r < 0) return fail(EDDSA_B200_EINVAL, "getrandom failed: %s", strerror(errno));
+        got += (size_t)r;
+    }
+    return 0;
+}
+
+int ed25519_verify_zip215_batched(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                                  const size_t *off, size_t fixed_len, const uint8_t *seed)
+{
+    uint8_t sd[32];
+    edg_job_t j = {OP_VERIFY, n, 2, {sig, pub, NULL}, {64, 32, 0}, 1, msgs, off, fixed_len, ok, 1, EDG_VERIFY_BATCHED, sd};
+    int rc = batched_seed(sd, seed);
+    if (!rc) rc = run_job(&j);
+    explicit_bzero(sd, sizeof sd);
+    return rc;
 }
 
 int ed25519_verify_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
@@ -753,25 +799,25 @@ int ed25519_verify_batch(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_
 
 int x25519_batch(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point)
 {
-    edg_job_t j = {OP_X25519, n, 2, {scalar, point, NULL}, {32, 32, 0}, 0, NULL, NULL, 0, out, 32, 0};
+    edg_job_t j = {OP_X25519, n, 2, {scalar, point, NULL}, {32, 32, 0}, 0, NULL, NULL, 0, out, 32, 0, NULL};
     return run_job(&j);
 }
 
 int x25519_base_batch(size_t n, uint8_t *out, const uint8_t *scalar)
 {
-    edg_job_t j = {OP_X25519_BASE, n, 1, {scalar, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0};
+    edg_job_t j = {OP_X25519_BASE, n, 1, {scalar, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0, NULL};
     return run_job(&j);
 }
 
 int pk_ed25519_to_x25519_batch(size_t n, uint8_t *out, const uint8_t *in)
 {
-    edg_job_t j = {OP_PK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0};
+    edg_job_t j = {OP_PK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0, NULL};
     return run_job(&j);
 }
 
 int sk_ed25519_to_x25519_batch(size_t n, uint8_t *out, const uint8_t *in)
 {
-    edg_job_t j = {OP_SK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0};
+    edg_job_t j = {OP_SK_CONV, n, 1, {in, NULL, NULL}, {32, 0, 0}, 0, NULL, NULL, 0, out, 32, 0, NULL};
     return run_job(&j);
 }
 
@@ -780,7 +826,7 @@ int sk_ed25519_to_x25519_batch(size_t n, uint8_t *out, const uint8_t *in)
  * items); a, b, out: n x 32 bytes, any 256-bit values */
 int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, int op)
 {
-    edg_job_t j = {OP_FE_TEST, n, 2, {a, b, NULL}, {32, 32, 0}, 0, NULL, NULL, (size_t)op, out, 32, 0};
+    edg_job_t j = {OP_FE_TEST, n, 2, {a, b, NULL}, {32, 32, 0}, 0, NULL, NULL, (size_t)op, out, 32, 0, NULL};
     return run_job(&j);
 }
 
@@ -790,7 +836,7 @@ int eddsa_b200_fe_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8
  * 2^(16 k), the signed 16-bit digits of a < 2^253 as the verify loop reads them); a, b, c, out: n x 32 bytes */
 int eddsa_b200_sc_selftest(size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *c, int op)
 {
-    edg_job_t j = {OP_SC_TEST, n, 3, {a, b, c}, {32, 32, 32}, 0, NULL, NULL, (size_t)op, out, 32, 0};
+    edg_job_t j = {OP_SC_TEST, n, 3, {a, b, c}, {32, 32, 32}, 0, NULL, NULL, (size_t)op, out, 32, 0, NULL};
     return run_job(&j);
 }
 
@@ -852,7 +898,7 @@ size_t eddsa_b200_debug_peek_staging(int which, int slot, uint8_t *out, size_t l
 static int misaligned(const void *p) { return ((uintptr_t)p & 15) != 0; }
 
 static int dev_call(edg_op_t op, size_t n, uint8_t *out, const uint8_t *a, const uint8_t *b, const uint8_t *msgs,
-                    const uint64_t *off, size_t fixed_len, int policy, void *stream)
+                    const uint64_t *off, size_t fixed_len, int policy, const uint8_t *seed, void *stream)
 {
     edg_dev_t *c;
     uint8_t *d_in[3] = {(uint8_t *)a, (uint8_t *)b, NULL};
@@ -864,19 +910,19 @@ static int dev_call(edg_op_t op, size_t n, uint8_t *out, const uint8_t *a, const
         return fail(EDDSA_B200_EINVAL, "device arrays must be non-NULL and 16-byte aligned");
     if ((op == OP_SIGN || op == OP_VERIFY) && !msgs && (off || fixed_len))
         return fail(EDDSA_B200_EINVAL, "NULL message blob");
-    return launch(c, op, n, out, d_in, msgs, (const unsigned long long *)off, fixed_len, policy, stream);
+    return launch(c, op, n, out, d_in, msgs, (const unsigned long long *)off, fixed_len, policy, seed, stream);
 }
 
 int ed25519_genpub_batch_dev(size_t n, uint8_t *pub, const uint8_t *sec, void *stream)
 {
-    return dev_call(OP_GENPUB, n, pub, sec, NULL, NULL, NULL, 0, 0, stream);
+    return dev_call(OP_GENPUB, n, pub, sec, NULL, NULL, NULL, 0, 0, NULL, stream);
 }
 
 int ed25519_sign_batch_dev(size_t n, uint8_t *sig, const uint8_t *sec, const uint8_t *pub, const uint8_t *msgs,
                            const uint64_t *off, size_t fixed_len, void *stream)
 {
     if (n && !pub) return fail(EDDSA_B200_EINVAL, "NULL pub array");
-    return dev_call(OP_SIGN, n, sig, sec, pub, msgs, off, fixed_len, 0, stream);
+    return dev_call(OP_SIGN, n, sig, sec, pub, msgs, off, fixed_len, 0, NULL, stream);
 }
 
 int ed25519_verify_policy_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
@@ -884,7 +930,18 @@ int ed25519_verify_policy_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, c
 {
     if (bad_policy(policy)) return EDDSA_B200_EINVAL;
     if (n && !pub) return fail(EDDSA_B200_EINVAL, "NULL pub array");
-    return dev_call(OP_VERIFY, n, ok, sig, pub, msgs, off, fixed_len, policy, stream);
+    return dev_call(OP_VERIFY, n, ok, sig, pub, msgs, off, fixed_len, policy, NULL, stream);
+}
+
+int ed25519_verify_zip215_batched_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                                      const uint64_t *off, size_t fixed_len, const uint8_t *seed, void *stream)
+{
+    uint8_t sd[32];
+    int rc = batched_seed(sd, seed);
+    if (!rc && n && !pub) rc = fail(EDDSA_B200_EINVAL, "NULL pub array");
+    if (!rc) rc = dev_call(OP_VERIFY, n, ok, sig, pub, msgs, off, fixed_len, EDG_VERIFY_BATCHED, sd, stream);
+    explicit_bzero(sd, sizeof sd);
+    return rc;
 }
 
 int ed25519_verify_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
@@ -896,22 +953,22 @@ int ed25519_verify_batch_dev(size_t n, uint8_t *ok, const uint8_t *sig, const ui
 int x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, const uint8_t *point, void *stream)
 {
     if (n && !point) return fail(EDDSA_B200_EINVAL, "NULL point array");
-    return dev_call(OP_X25519, n, out, scalar, point, NULL, NULL, 0, 0, stream);
+    return dev_call(OP_X25519, n, out, scalar, point, NULL, NULL, 0, 0, NULL, stream);
 }
 
 int x25519_base_batch_dev(size_t n, uint8_t *out, const uint8_t *scalar, void *stream)
 {
-    return dev_call(OP_X25519_BASE, n, out, scalar, NULL, NULL, NULL, 0, 0, stream);
+    return dev_call(OP_X25519_BASE, n, out, scalar, NULL, NULL, NULL, 0, 0, NULL, stream);
 }
 
 int pk_ed25519_to_x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *in, void *stream)
 {
-    return dev_call(OP_PK_CONV, n, out, in, NULL, NULL, NULL, 0, 0, stream);
+    return dev_call(OP_PK_CONV, n, out, in, NULL, NULL, NULL, 0, 0, NULL, stream);
 }
 
 int sk_ed25519_to_x25519_batch_dev(size_t n, uint8_t *out, const uint8_t *in, void *stream)
 {
-    return dev_call(OP_SK_CONV, n, out, in, NULL, NULL, NULL, 0, 0, stream);
+    return dev_call(OP_SK_CONV, n, out, in, NULL, NULL, NULL, 0, 0, NULL, stream);
 }
 
 /* ---------------------------------------------------------------------------------------------

@@ -12,6 +12,7 @@
 // Also hosts pk_ed25519_to_x25519 (it shares the decompression).
 // Replaces ed25519_verify / pk_ed25519_to_x25519: /root/reference/lib/ed25519-sha512.c:148-237.
 #define EDG_SHA_MSGWORD_NOINLINE
+#include <string.h>
 #include "kernel_common.cuh"
 using namespace edg;
 
@@ -37,6 +38,7 @@ using namespace edg;
 namespace {
 constexpr int kVThreads = EDG_VTHREADS;
 constexpr int kMsgTile = EDG_MSG_TILE;
+static_assert(EDG_VBATCH_K == 4 || EDG_VBATCH_K == 8 || EDG_VBATCH_K == 16, "batch rows: 4, 8 or 16");
 constexpr int kMsgTileBits = kMsgTile == 512 ? 9 : kMsgTile == 1024 ? 10 : kMsgTile == 2048 ? 11 : 12;
 static_assert(kMsgTile == (1 << kMsgTileBits), "tile size must be a power of two between 512 and 4096");
 
@@ -47,14 +49,17 @@ static_assert(kMsgTile == (1 << kMsgTileBits), "tile size must be a power of two
 #define EDG_NWIN_SPLIT 33
 
 // scalars half for signature k of the pass (record k); callable from diverged code (lanes group by __activemask)
+// BATCHED: also the side record of the batched ZIP215 check (side + k * EDG_VSIDE_WORDS, weights from seed)
+template <bool BATCHED = false>
 __device__ __forceinline__ void verify_scalars_of(size_t n, size_t k, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                                                   const unsigned long long *off, unsigned long long fixed_len, u32 *state,
-                                                  unsigned int *perm, unsigned int *counters, int full_scalars) {
+                                                  unsigned int *perm, unsigned int *counters, int full_scalars, u32 *side = 0,
+                                                  const verify_seed &seed = {}) {
     const uint8_t *m; u64 len;
     msg_of(m, len, msgs, off, fixed_len, k);
     const u32 *sg = reinterpret_cast<const u32 *>(sig + 64 * k), *pk = reinterpret_cast<const u32 *>(pub + 32 * k);
     verify_scalars v;
-    const int nwin = ed25519_verify_front_scalars(v, sg, pk, m, len, full_scalars != 0);
+    const int nwin = ed25519_verify_front_scalars<BATCHED>(v, sg, pk, m, len, full_scalars != 0, side + k * EDG_VSIDE_WORDS, &seed);
     ed25519_verify_store_scalars(state + k * EDG_VSTATE_WORDS, v, nwin);
     const unsigned active = __activemask();
     const unsigned lane = threadIdx.x & 31u, leader = __ffs(active) - 1;
@@ -72,13 +77,18 @@ __device__ __forceinline__ void verify_scalars_of(size_t n, size_t k, const uint
 }
 
 // the scalars half (RAGGED: the batch has an offsets array — tiles of kMsgTile signatures sorted by message length)
-template <bool RAGGED>
+// BATCHED: the batched ZIP215 check's instantiation, which also writes the side records; side... is then (u32 *side,
+// verify_seed seed), and empty otherwise (the per-signature instantiations keep their parameter list)
+template <bool RAGGED, bool BATCHED = false, class... Side>
 __global__ void __launch_bounds__(kThreads, EDG_LB_VERIFY) k_verify_scalars(size_t n, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
                                                        const unsigned long long *off, unsigned long long fixed_len, u32 *state,
-                                                       unsigned int *perm, unsigned int *counters, int full_scalars) {
+                                                       unsigned int *perm, unsigned int *counters, int full_scalars, Side... side) {
     if constexpr (!RAGGED) {
         const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-        if (k < n) verify_scalars_of(n, k, sig, pub, msgs, off, fixed_len, state, perm, counters, full_scalars);
+        if (k < n) {
+            if constexpr (BATCHED) verify_scalars_of<true>(n, k, sig, pub, msgs, off, fixed_len, state, perm, counters, full_scalars, side...);
+            else verify_scalars_of(n, k, sig, pub, msgs, off, fixed_len, state, perm, counters, full_scalars);
+        }
     } else {
         __shared__ u32 s_key[kMsgTile];
         for (size_t t0 = (size_t)blockIdx.x * kMsgTile; t0 < n; t0 += (size_t)gridDim.x * kMsgTile) {
@@ -88,7 +98,11 @@ __global__ void __launch_bounds__(kThreads, EDG_LB_VERIFY) k_verify_scalars(size
             for (int e = threadIdx.x; e < kMsgTile; e += blockDim.x) {
                 const u32 key = s_key[e];
                 if (key == 0xffffffffu) break;
-                verify_scalars_of(n, t0 + (key & (kMsgTile - 1)), sig, pub, msgs, off, fixed_len, state, perm, counters, full_scalars);
+                if constexpr (BATCHED)
+                    verify_scalars_of<true>(n, t0 + (key & (kMsgTile - 1)), sig, pub, msgs, off, fixed_len, state, perm, counters, full_scalars,
+                                            side...);
+                else
+                    verify_scalars_of(n, t0 + (key & (kMsgTile - 1)), sig, pub, msgs, off, fixed_len, state, perm, counters, full_scalars);
             }
         }
     }
@@ -111,6 +125,55 @@ __global__ void __launch_bounds__(kVThreads, EDG_LB_VLOOP) k_verify(size_t n, ui
     const unsigned k = perm[j < n ? j : n - 1];
     __shared__ uint4 s_stage[16 * kVThreads];                  // 2 table entries x 8 x 16 bytes per thread, chunk-major
     const u32 r = ed25519_verify_loop<COFACTORED>(state + (size_t)k * EDG_VSTATE_WORDS, wtab, reinterpret_cast<u32 *>(s_stage));
+    if (j < n) ok[k] = (uint8_t)r;
+}
+
+// The batched ZIP215 check (ops.cuh: ed25519_verify_batched_loop).  Warp w covers rows [32 K w, 32 K (w + 1)); lane l
+// checks rows 32 K w + l + 32 r, r < K.  A lane whose equation holds writes ok = flag bit 0 for its rows; a lane whose
+// equation fails appends its rows to list (count: *count, one atomic per warp), or, with no_fallback (test hook), writes 0.
+template <int K>
+__global__ void __launch_bounds__(kVThreads, EDG_LB_VLOOP) k_verify_batched(size_t n, uint8_t *ok, const u32 *state, const u32 *side,
+                                                                           const u32 *__restrict__ wtab, unsigned int *list, unsigned int *count,
+                                                                           int no_fallback) {
+    const size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x, w = g >> 5, lane = g & 31;
+    if (32 * K * w >= n) return;                          // whole warps
+    const size_t first = 32 * K * w + lane;
+    int cnt = 0;
+    u32 incl = 0;
+#pragma unroll
+    for (int r = 0; r < K; r++) {
+        const size_t row = first + 32 * r;
+        if (row < n) { cnt = r + 1; incl |= (state[row * EDG_VSTATE_WORDS + 600] & 1u) << r; }
+    }
+    const size_t r0 = cnt ? first : n - 1;                // a lane without rows adds identity entries of the last row
+    const u32 holds = ed25519_verify_batched_loop<K>(state + r0 * EDG_VSTATE_WORDS, side + r0 * EDG_VSIDE_WORDS, 32, cnt ? cnt : 1, incl, wtab);
+    const bool fail = !holds && !no_fallback;
+    if (!fail)
+        for (int r = 0; r < cnt; r++) ok[first + 32 * r] = (uint8_t)(holds & (incl >> r) & 1u);
+    unsigned b[K], total = 0;                             // row r of the failing lanes goes after row r - 1 of all of them
+#pragma unroll
+    for (int r = 0; r < K; r++) { b[r] = __ballot_sync(0xffffffffu, fail && r < cnt); total += __popc(b[r]); }
+    if (total == 0) return;
+    unsigned base = 0;
+    if (lane == 0) base = atomicAdd(count, total);
+    base = __shfl_sync(0xffffffffu, base, 0);
+    const unsigned below = (1u << lane) - 1u;
+#pragma unroll
+    for (int r = 0; r < K; r++) {
+        if ((b[r] >> lane) & 1u) list[base + __popc(b[r] & below)] = (unsigned)(first + 32 * r);
+        base += __popc(b[r]);
+    }
+}
+
+// The per-signature ZIP215 loop over the rows of failed batch equations: list[0 .. *count).  The grid covers the worst
+// case (every row); blocks past the count exit.  Whole warps stay together as in k_verify.
+__global__ void __launch_bounds__(kVThreads, EDG_LB_VLOOP) k_verify_list(uint8_t *ok, const u32 *state, const unsigned int *list,
+                                                                        const unsigned int *count, const u32 *__restrict__ wtab) {
+    const size_t n = *count, j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if ((j & ~(size_t)31) >= n) return;
+    const unsigned k = list[j < n ? j : n - 1];
+    __shared__ uint4 s_stage[16 * kVThreads];
+    const u32 r = ed25519_verify_loop<true>(state + (size_t)k * EDG_VSTATE_WORDS, wtab, reinterpret_cast<u32 *>(s_stage));
     if (j < n) ok[k] = (uint8_t)r;
 }
 
@@ -138,6 +201,7 @@ __global__ void __launch_bounds__(kThreads) k_pk_convert(size_t n, uint8_t *out,
 
 int g_waves = EDG_VERIFY_WAVES;
 int g_full_scalars = 0;
+int g_no_fallback = 0;
 
 }  // namespace
 
@@ -159,6 +223,11 @@ size_t edg_verify_record_bytes(void) { return EDG_VSTATE_WORDS * sizeof(u32); }
 static size_t perm_offset(size_t records) { return records * EDG_VSTATE_WORDS * sizeof(u32); }
 static size_t counters_offset(size_t records) { return perm_offset(records) + ((records * sizeof(unsigned) + 255) & ~(size_t)255); }
 size_t edg_verify_scratch_bytes(size_t records) { return counters_offset(records) + 256; }
+
+// the batched ZIP215 check adds the side records (EDG_VSIDE_WORDS words per row) and the list of rows to re-check
+static size_t side_offset(size_t records) { return edg_verify_scratch_bytes(records); }
+static size_t list_offset(size_t records) { return side_offset(records) + records * EDG_VSIDE_WORDS * sizeof(u32); }
+size_t edg_verify_batched_scratch_bytes(size_t records) { return list_offset(records) + ((records * sizeof(unsigned) + 255) & ~(size_t)255); }
 
 size_t edg_verify_table_bytes(void) { return (2 * (size_t)EDG_WTAB_WORDS + 48) * sizeof(u32); }
 
@@ -207,6 +276,49 @@ int edg_launch_verify_policy(size_t n, uint8_t *ok, const uint8_t *sig, const ui
         }
         loop<<<(unsigned)((m + kVThreads - 1) / kVThreads), kVThreads, 0, st>>>(m, ok + first, state, perm, (const u32 *)table);
     }
+    return (int)cudaGetLastError();
+}
+
+// test hook (EDDSA_B200_DEBUG_NO_FALLBACK=1): a failing batch equation writes 0 to its rows, nothing is re-checked
+void edg_verify_debug_no_fallback(int on) { g_no_fallback = on; }
+
+// scratch: edg_verify_batched_scratch_bytes(records) bytes; seed: 32 bytes in host memory (passed to the scalars kernel by value)
+int edg_launch_verify_batched(size_t n, uint8_t *ok, const uint8_t *sig, const uint8_t *pub, const uint8_t *msgs,
+                              const unsigned long long *off, unsigned long long fixed_len, const uint8_t *seed, void *scratch, size_t records,
+                              const void *table, int sm_count, void *stream, unsigned *launches) {
+    cudaStream_t st = (cudaStream_t)stream;
+    u32 *state = (u32 *)scratch, *side = (u32 *)((uint8_t *)scratch + side_offset(records));
+    unsigned int *perm = (unsigned int *)((uint8_t *)scratch + perm_offset(records));
+    unsigned int *counters = (unsigned int *)((uint8_t *)scratch + counters_offset(records));
+    unsigned int *list = (unsigned int *)((uint8_t *)scratch + list_offset(records));
+    const u32 *wtab = (const u32 *)table;
+    constexpr int K = EDG_VBATCH_K;
+    if (records == 0) return (int)cudaErrorInvalidValue;
+    verify_seed sd;
+    memcpy(sd.w, seed, sizeof sd.w);                      // little-endian host
+    for (size_t first = 0; first < n; first += records) {
+        const size_t m = n - first < records ? n - first : records;
+        const unsigned nb = (unsigned)((m + kThreads - 1) / kThreads);
+        const uint8_t *sg = sig + 64 * first, *pk = pub + 32 * first;
+        cudaMemsetAsync(counters, 0, 3 * sizeof(unsigned int), st);
+        if (off) {
+            int bps = 0;
+            grid_for(k_verify_scalars<true, true, u32 *, verify_seed>, m, 0, sm_count, &bps);
+            const size_t tiles = (m + kMsgTile - 1) / kMsgTile, cap = (size_t)sm_count * bps;
+            k_verify_scalars<true, true, u32 *, verify_seed><<<(unsigned)(tiles < cap ? tiles : cap), kThreads, 0, st>>>(m, sg, pk, msgs, off + first, fixed_len, state, perm,
+                                                                                                   counters, g_full_scalars, side, sd);
+        } else {
+            k_verify_scalars<false, true, u32 *, verify_seed><<<nb, kThreads, 0, st>>>(m, sg, pk, msgs + first * fixed_len, nullptr, fixed_len, state, perm, counters,
+                                                                  g_full_scalars, side, sd);
+        }
+        k_verify_points<EDG_VERIFY_ZIP215><<<nb, kThreads, 0, st>>>(m, sg, pk, state);
+        const size_t warps = (m + 32 * K - 1) / (32 * K);
+        k_verify_batched<K><<<(unsigned)((32 * warps + kVThreads - 1) / kVThreads), kVThreads, 0, st>>>(m, ok + first, state, side, wtab, list,
+                                                                                                      counters + 2, g_no_fallback);
+        k_verify_list<<<(unsigned)((m + kVThreads - 1) / kVThreads), kVThreads, 0, st>>>(ok + first, state, list, counters + 2, wtab);
+        *launches += 4;
+    }
+    memset(&sd, 0, sizeof sd);
     return (int)cudaGetLastError();
 }
 

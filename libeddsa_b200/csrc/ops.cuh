@@ -461,7 +461,13 @@ EDG_HD int sc_digit16(const u32 *e, int j) { return (int)((e[j >> 3] >> (4 * (j 
 // front, scalars: returns the number of windows this signature needs.
 struct verify_scalars { u32 et[8], er[8], es[8], rho_neg; };
 
-EDG_HD int ed25519_verify_front_scalars(verify_scalars &v, const u32 *sig, const u32 *pub, const uint8_t *msg, u64 len, bool full_scalars = false) {
+struct verify_seed { u32 w[8]; };                       // the 32 seed bytes of a batched call, little-endian words
+EDG_HD void ed25519_verify_side_record(u32 *side, const verify_seed &seed, const u32 t[8], const u32 sraw[8], const u32 s[8]);
+
+// SIDE (batched ZIP215): also writes the row's side record (ed25519_verify_side_record) to side.
+template <bool SIDE = false>
+EDG_HD int ed25519_verify_front_scalars(verify_scalars &v, const u32 *sig, const u32 *pub, const uint8_t *msg, u64 len, bool full_scalars = false,
+                                        u32 *side = 0, const verify_seed *seed = 0) {
     // t = H(R || A || M) mod L, bytes exactly as given (Q4)                                    :166-171
     u64 pre[8], st[8];
     u32 h[16], t[8], s[8];
@@ -478,6 +484,7 @@ EDG_HD int ed25519_verify_front_scalars(verify_scalars &v, const u32 *sig, const
     half_gcd(v.er, v.rho_neg, v.et, t, full_scalars);     // er = |rho|, et = tau  (full_scalars: (1, t), the fallback)
     load_words8(h, sig + 8);
     sc_reduce256(s, h);                                   // no range check on S (Q1)               :163
+    if constexpr (SIDE) ed25519_verify_side_record(side, *seed, t, h, s);
 #pragma unroll
     for (int i = 0; i < 8; i++) h[i] = 0;
     sc_muladd(v.es, v.er, s, h);                          // |rho| S mod L
@@ -537,6 +544,100 @@ EDG_HD void ed25519_verify_front(u32 *state, const u32 *sig, const u32 *pub, con
     ed25519_verify_front_points<POLICY>(state, sig, pub);
 }
 
+// One step of the verify window loops, as a macro so that both loops share it without any change to the code the
+// per-signature loop compiles to: a doubling (step < 4), the addition of a cached entry of a point table (step 4, 5:
+// CACHED(q, neg) declares and loads ge_cached q and the u32 mask neg, all-ones when the entry is to be negated) or of an
+// affine window-table entry (step >= 6: BASE(q) declares and loads ge_pre q).  Doubling and addition end in the same
+// four products (X3 = E F, Y3 = G H, Z3 = F G, T3 = E H): sharing that tail keeps the loops inside the instruction cache.
+// NEED_T: an addition follows, so T3 is computed.  Public data only: the field operations are the pub_ flavour (fe.cuh),
+// in groups of independent operations whose pending carries are settled by one rarely taken branch per group.
+#define EDG_VERIFY_STEP(R, step, NEED_T, CACHED, BASE)                                                                              \
+    {                                                                                                                               \
+        fe e, f, g, h;                                                                                                              \
+        bool p0, p1, p2, p3;                                                                                                        \
+        if (step < 4) {                               /* doubling prologue                 [ed_double, ed.c:211] */                 \
+            fe a, b, c, s;                                                                                                          \
+            p0 = pub_sq(a, R.X);                                                                                                    \
+            p1 = pub_sq(b, R.Y);                                                                                                    \
+            p2 = pub_sq(c, R.Z);                                                                                                    \
+            p3 = pub_add(s, R.X, R.Y);                                                                                              \
+            if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(a, p0); pub_settle_add(b, p1); pub_settle_add(c, p2); pub_settle_add(s, p3); } \
+            p0 = pub_dbl(c, c);                                                                                                     \
+            p1 = pub_sq(s, s);                                                                                                      \
+            p2 = pub_add(h, a, b);                                                                                                  \
+            p3 = pub_sub(g, a, b);                                                                                                  \
+            if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(c, p0); pub_settle_add(s, p1); pub_settle_add(h, p2); pub_settle_sub(g, p3); } \
+            p0 = pub_sub(e, h, s);                                                                                                  \
+            p1 = pub_add(f, c, g);                                                                                                  \
+            if (pub_rare(p0 | p1)) { pub_settle_sub(e, p0); pub_settle_add(f, p1); }                                               \
+        } else {                                      /* addition prologue   [ed_add ed.c:175 / ed_add_pc :282] */                 \
+            fe ypx, ymx, t2d, a, b, c, d;                                                                                           \
+            if (step < 6) {                           /* cached entry of a point table */                                          \
+                CACHED(q, neg)                                                                                                      \
+                fe nt;                                /* q = neg ? -q : q  (ge_cached_cneg, negation in the group below) */        \
+                fe_cswap(q.ypx, q.ymx, neg);                                                                                        \
+                fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx);                                                                           \
+                p0 = pub_neg(nt, q.t2d);                                                                                            \
+                p1 = pub_mul(d, R.Z, q.z2);                                                                                         \
+                p2 = pub_sub(a, R.Y, R.X);                                                                                          \
+                p3 = pub_add(b, R.Y, R.X);                                                                                          \
+                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_sub(nt, p0); pub_settle_add(d, p1); pub_settle_sub(a, p2); pub_settle_add(b, p3); } \
+                fe_select(t2d, q.t2d, nt, neg);                                                                                     \
+            } else {                                  /* affine entry of a window table (Z2 = 1) */                                \
+                BASE(q)                                                                                                             \
+                fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx); fe_copy(t2d, q.xy2d);                                                     \
+                p0 = pub_dbl(d, R.Z);                                                                                               \
+                p2 = pub_sub(a, R.Y, R.X);                                                                                          \
+                p3 = pub_add(b, R.Y, R.X);                                                                                          \
+                if (pub_rare(p0 | p2 | p3)) { pub_settle_add(d, p0); pub_settle_sub(a, p2); pub_settle_add(b, p3); }              \
+            }                                                                                                                       \
+            p0 = pub_mul(a, a, ymx);                                                                                                \
+            p1 = pub_mul(b, b, ypx);                                                                                                \
+            p2 = pub_mul(c, R.T, t2d);                                                                                              \
+            if (pub_rare(p0 | p1 | p2)) { pub_settle_add(a, p0); pub_settle_add(b, p1); pub_settle_add(c, p2); }                  \
+            p0 = pub_sub(e, b, a);                                                                                                  \
+            p1 = pub_sub(f, d, c);                                                                                                  \
+            p2 = pub_add(g, d, c);                                                                                                  \
+            p3 = pub_add(h, b, a);                                                                                                  \
+            if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_sub(e, p0); pub_settle_sub(f, p1); pub_settle_add(g, p2); pub_settle_add(h, p3); } \
+        }                                                                                                                           \
+        p0 = pub_mul(R.X, e, f);                      /* shared tail */                                                            \
+        p1 = pub_mul(R.Y, g, h);                                                                                                    \
+        p2 = pub_mul(R.Z, f, g);                                                                                                    \
+        p3 = false;                                                                                                                 \
+        if (NEED_T) p3 = pub_mul(R.T, e, h);                                                                                        \
+        if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(R.X, p0); pub_settle_add(R.Y, p1); pub_settle_add(R.Z, p2); pub_settle_add(R.T, p3); } \
+    }
+
+// ed25519_verify_loop's entry loads: digit j of tau (step 4, Q = -A, sign flipped by rho_neg) or |rho| (step 5, P = -R')
+// from the thread's own record, or from the shared-memory staging area when stage is set (device only); 16-bit digit of
+// rho S from the tables of B (step 6) and 2^128 B (step 7).
+#if defined(__CUDA_ARCH__)
+#define EDG_VLOOP_STAGED(q)                                                                                                         \
+    if (stage) {                                                                                                                    \
+        if (step == 4) asm volatile("cp.async.wait_group 0;" ::: "memory");     /* this thread's own copies only */                 \
+        const uint4 *sp = reinterpret_cast<const uint4 *>(stage) + threadIdx.x + (step == 4 ? 0 : 8) * blockDim.x;                  \
+        u32 w[32];                                                                                                                  \
+        _Pragma("unroll") for (int c = 0; c < 8; c++) { const uint4 v = sp[c * blockDim.x]; w[4 * c] = v.x; w[4 * c + 1] = v.y; w[4 * c + 2] = v.z; w[4 * c + 3] = v.w; } \
+        _Pragma("unroll") for (int i = 0; i < 8; i++) { q.ypx.v[i] = w[i]; q.ymx.v[i] = w[8 + i]; q.z2.v[i] = w[16 + i]; q.t2d.v[i] = w[24 + i]; } \
+    } else
+#else
+#define EDG_VLOOP_STAGED(q)
+#endif
+#define EDG_VLOOP_CACHED(q, neg)                                                                                                    \
+    const int dg = sc_digit16(step == 4 ? et : er, j);                                                                              \
+    const u32 sgn = (u32)(dg >> 31);                                                                                                \
+    const u32 absd = ((u32)dg ^ sgn) - sgn;                                                                                         \
+    const u32 neg = step == 4 ? sgn ^ rho_neg : sgn;                                                                                \
+    ge_cached q;                                                                                                                    \
+    EDG_VLOOP_STAGED(q)                                                                                                             \
+    ge_cached_load(q, qtab + (step == 4 ? 0 : 288) + 32 * absd);
+#define EDG_VLOOP_BASE(q)                                                                                                           \
+    const int k = (j >> 2) + (step == 6 ? 0 : 8);                                                                                   \
+    const int ds = (int)((es[k >> 1] >> (16 * (k & 1))) & 0xffffu) - 0x8000;                                                        \
+    ge_pre q;                                                                                                                       \
+    ge_pre_load_wtab(q, wtab + (step == 6 ? 0u : EDG_WTAB_WORDS), ds);
+
 // stage (device only, may be null): this block's shared-memory staging area, 16 chunks x blockDim.x threads x 16 bytes.
 // At the start of a window every thread starts asynchronous copies (cp.async, no registers involved) of the two
 // table entries the window will add; they arrive while the four doublings run, so the additions find them in
@@ -562,11 +663,9 @@ EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0
     sc_recode_radix16_n(er, nwin);
     const u32 *qtab = state;
 
-    // Straus main loop.  Each 4-bit window is up to eight steps through ONE loop body — four doublings, the
-    // additions of the two scratch-table entries and, every fourth window below bit 128, of the two base-table
-    // entries — because doubling and addition end in the same four products (X3 = E F, Y3 = G H, Z3 = F G,
-    // T3 = E H): sharing that tail keeps the loop inside the instruction cache.  T3 is only computed when an
-    // addition follows.
+    // Straus main loop.  Each 4-bit window is up to eight steps through ONE loop body (EDG_VERIFY_STEP) — four
+    // doublings, the additions of the two scratch-table entries and, every fourth window below bit 128, of the two
+    // base-table entries.  T3 is only computed when an addition follows.
     ge_p3 R;
     ge_identity(R);
 #pragma unroll 1
@@ -588,86 +687,109 @@ EDG_HD u32 ed25519_verify_loop(const u32 *state, const u32 *wtab, u32 *stage = 0
 #endif
 #pragma unroll 1
         for (int step = (j == nwin - 1 ? 4 : 0); step < last; step++) {
-            // Public data only: the field operations are the pub_ flavour (fe.cuh), in groups of independent operations
-            // whose pending carries are settled by one rarely taken branch per group.
-            fe e, f, g, h;
-            bool p0, p1, p2, p3;
-            if (step < 4) {                                   // doubling prologue                 [ed_double, ed.c:211]
-                fe a, b, c, s;
-                p0 = pub_sq(a, R.X);
-                p1 = pub_sq(b, R.Y);
-                p2 = pub_sq(c, R.Z);
-                p3 = pub_add(s, R.X, R.Y);
-                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(a, p0); pub_settle_add(b, p1); pub_settle_add(c, p2); pub_settle_add(s, p3); }
-                p0 = pub_dbl(c, c);
-                p1 = pub_sq(s, s);
-                p2 = pub_add(h, a, b);
-                p3 = pub_sub(g, a, b);
-                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(c, p0); pub_settle_add(s, p1); pub_settle_add(h, p2); pub_settle_sub(g, p3); }
-                p0 = pub_sub(e, h, s);
-                p1 = pub_add(f, c, g);
-                if (pub_rare(p0 | p1)) { pub_settle_sub(e, p0); pub_settle_add(f, p1); }
-            } else {                                          // addition prologue                 [ed_add ed.c:175 / ed_add_pc :282]
-                fe ypx, ymx, t2d, a, b, c, d;
-                if (step < 6) {                               // digit * Q or digit * P: cached entry from this thread's scratch
-                    const int dg = sc_digit16(step == 4 ? et : er, j);
-                    const u32 sgn = (u32)(dg >> 31);
-                    const u32 absd = ((u32)dg ^ sgn) - sgn;
-                    const u32 neg = step == 4 ? sgn ^ rho_neg : sgn;
-                    ge_cached q;
-#if defined(__CUDA_ARCH__)
-                    if (stage) {
-                        if (step == 4) asm volatile("cp.async.wait_group 0;" ::: "memory");     // this thread's own copies only
-                        const uint4 *sp = reinterpret_cast<const uint4 *>(stage) + threadIdx.x + (step == 4 ? 0 : 8) * blockDim.x;
-                        u32 w[32];
-#pragma unroll
-                        for (int c = 0; c < 8; c++) { const uint4 v = sp[c * blockDim.x]; w[4 * c] = v.x; w[4 * c + 1] = v.y; w[4 * c + 2] = v.z; w[4 * c + 3] = v.w; }
-#pragma unroll
-                        for (int i = 0; i < 8; i++) { q.ypx.v[i] = w[i]; q.ymx.v[i] = w[8 + i]; q.z2.v[i] = w[16 + i]; q.t2d.v[i] = w[24 + i]; }
-                    } else
-#endif
-                    ge_cached_load(q, qtab + (step == 4 ? 0 : 288) + 32 * absd);
-                    fe nt;                                    // q = neg ? -q : q  (ge_cached_cneg, negation in the group below)
-                    fe_cswap(q.ypx, q.ymx, neg);
-                    fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx);
-                    p0 = pub_neg(nt, q.t2d);
-                    p1 = pub_mul(d, R.Z, q.z2);
-                    p2 = pub_sub(a, R.Y, R.X);
-                    p3 = pub_add(b, R.Y, R.X);
-                    if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_sub(nt, p0); pub_settle_add(d, p1); pub_settle_sub(a, p2); pub_settle_add(b, p3); }
-                    fe_select(t2d, q.t2d, nt, neg);
-                } else {                                      // digit * B or digit * 2^128 B: affine entry of a window table (Z2 = 1)
-                    const int k = (j >> 2) + (step == 6 ? 0 : 8);
-                    const int ds = (int)((es[k >> 1] >> (16 * (k & 1))) & 0xffffu) - 0x8000;
-                    ge_pre q;
-                    ge_pre_load_wtab(q, wtab + (step == 6 ? 0u : EDG_WTAB_WORDS), ds);
-                    fe_copy(ypx, q.ypx); fe_copy(ymx, q.ymx); fe_copy(t2d, q.xy2d);
-                    p0 = pub_dbl(d, R.Z);
-                    p2 = pub_sub(a, R.Y, R.X);
-                    p3 = pub_add(b, R.Y, R.X);
-                    if (pub_rare(p0 | p2 | p3)) { pub_settle_add(d, p0); pub_settle_sub(a, p2); pub_settle_add(b, p3); }
-                }
-                p0 = pub_mul(a, a, ymx);
-                p1 = pub_mul(b, b, ypx);
-                p2 = pub_mul(c, R.T, t2d);
-                if (pub_rare(p0 | p1 | p2)) { pub_settle_add(a, p0); pub_settle_add(b, p1); pub_settle_add(c, p2); }
-                p0 = pub_sub(e, b, a);
-                p1 = pub_sub(f, d, c);
-                p2 = pub_add(g, d, c);
-                p3 = pub_add(h, b, a);
-                if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_sub(e, p0); pub_settle_sub(f, p1); pub_settle_add(g, p2); pub_settle_add(h, p3); }
-            }
-            p0 = pub_mul(R.X, e, f);                          // shared tail
-            p1 = pub_mul(R.Y, g, h);
-            p2 = pub_mul(R.Z, f, g);
-            p3 = false;
-            if (step == 3 || step == 4 || step == 6 || (step == 5 && has_b)) p3 = pub_mul(R.T, e, h);
-            if (pub_rare(p0 | p1 | p2 | p3)) { pub_settle_add(R.X, p0); pub_settle_add(R.Y, p1); pub_settle_add(R.Z, p2); pub_settle_add(R.T, p3); }
+            EDG_VERIFY_STEP(R, step, step == 3 || step == 4 || step == 6 || (step == 5 && has_b), EDG_VLOOP_CACHED, EDG_VLOOP_BASE)
         }
     }
     // the sum is the neutral element (0 : 1 : 1)  <=>  X = 0 and Y = Z   (Z != 0: the addition law is complete)
     const u32 is_o = fe_is_zero(R.X) & fe_eq(R.Y, R.Z);
     return is_o & (good & 1u);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Batched ZIP215 verification: one thread checks ONE random linear combination of K rows (K = EDG_VBATCH_K)
+//   8 ( (sum z_i S_i mod L) B  +  sum (z_i t_i mod L) (-A_i)  +  sum z_i (-R_i) ) == O
+// over the rows whose flag bit 0 is set (S < L, A and R on the curve), with weights z_i < 2^128 drawn from a per-call
+// seed.  The rows share one doubling chain, so a row costs 256 / K doublings instead of ~132.  If every included row
+// satisfies 8 D_i = O the equation holds; otherwise it holds with probability at most 2^-127 over the seed (DESIGN.md
+// §2), and a failing equation sends its rows to the per-signature loop.
+// ------------------------------------------------------------------------------------------------
+#ifndef EDG_VBATCH_K
+#define EDG_VBATCH_K 8      /* rows per batch equation (DESIGN.md §3.4 item 5: 4, 8 and 16 measured) */
+#endif
+// side record of a row (written by the scalars stage next to the record): [0, 8) z t mod L recoded to 64 signed 4-bit
+// digits, [8, 16) z recoded to 33 signed 4-bit digits (z < 2^128 needs the 33rd), [16, 24) z (S mod L) mod L
+#define EDG_VSIDE_WORDS 24
+
+// z = SHA-512(seed || t || S)[0..16) as a little-endian integer with bit 0 set: 0 < z < 2^128 < L.  t binds R, A and M, so
+// the weight of a row depends on its contents only (not on its position, pass or shard).  sraw: the signature's S bytes.
+EDG_HD void ed25519_verify_side_record(u32 *side, const verify_seed &seed, const u32 t[8], const u32 sraw[8], const u32 s[8]) {
+    u64 w[16], st[8];                                     // 96 bytes: one padded block
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        w[k] = be64_from_le_words(seed.w[2 * k], seed.w[2 * k + 1]);
+        w[4 + k] = be64_from_le_words(t[2 * k], t[2 * k + 1]);
+        w[8 + k] = be64_from_le_words(sraw[2 * k], sraw[2 * k + 1]);
+    }
+    w[12] = 0x8000000000000000ull; w[13] = 0; w[14] = 0; w[15] = 96 * 8;
+    sha512_iv(st);
+    sha512_compress(st, w);
+    u32 h[16], z[8], x[8], zero[8];
+    sha512_state_to_le_words(h, st);
+#pragma unroll
+    for (int i = 0; i < 8; i++) { z[i] = i < 4 ? h[i] : 0u; zero[i] = 0; }
+    z[0] |= 1u;
+    sc_muladd(x, z, t, zero);
+    sc_recode_radix16_n(x, 64);
+#pragma unroll
+    for (int i = 0; i < 8; i++) side[i] = x[i];
+    sc_muladd(x, z, s, zero);
+#pragma unroll
+    for (int i = 0; i < 8; i++) side[16 + i] = x[i];
+    sc_recode_radix16_n(z, 33);
+#pragma unroll
+    for (int i = 0; i < 8; i++) side[8 + i] = z[i];
+}
+
+// Entry loads of ed25519_verify_batched_loop: addition a = stp - 4 of the window adds digit j of z t (a < K, table of -A)
+// or of z (table of -R') of row a mod K; absent rows (r >= cnt) use row cnt - 1's identity entry, and rows outside incl
+// take digit 0 (the identity entry of their table).
+#define EDG_VBATCH_CACHED(q, neg)                                                                                                   \
+    const int a_ = stp - 4, r_ = a_ < K ? a_ : a_ - K, rr_ = r_ < cnt ? r_ : cnt - 1;                                                 \
+    const int dg = ((incl >> r_) & 1u) ? sc_digit16(side + (size_t)rr_ * stride * EDG_VSIDE_WORDS + (a_ < K ? 0 : 8), j) : 0;      \
+    const u32 neg = (u32)(dg >> 31);                                                                                                \
+    const u32 absd = ((u32)dg ^ neg) - neg;                                                                                         \
+    ge_cached q;                                                                                                                    \
+    ge_cached_load(q, state + (size_t)rr_ * stride * EDG_VSTATE_WORDS + (a_ < K ? 0 : 288) + 32 * absd);
+
+// One batch equation over K rows: row r's record at state + r stride EDG_VSTATE_WORDS and side record at
+// side + r stride EDG_VSIDE_WORDS, for r < cnt (1 <= cnt <= K); incl: bit r set when row r takes part (r < cnt and flag
+// bit 0 of its record).  Returns 1 when the equation holds.  64 signed 4-bit windows (the z t are full-size scalars); a
+// window j adds K entries of -A, K more of -R' when j < 33, and the digits of B and 2^128 B when j = 0 mod 4, j < 32.  Every
+// lane runs the same steps: the control flow is uniform across the warp.  Then three doublings (the cofactor) and the
+// comparison with the neutral element.
+template <int K>
+EDG_HD u32 ed25519_verify_batched_loop(const u32 *state, const u32 *side, size_t stride, int cnt, u32 incl, const u32 *wtab) {
+    u32 acc[16], es[8];                                   // sum of z S over the included rows (< K L < 2^257), then mod L
+#pragma unroll
+    for (int i = 0; i < 16; i++) acc[i] = 0;
+#pragma unroll 1
+    for (int r = 0; r < cnt; r++) {
+        const u32 *zs = side + (size_t)r * stride * EDG_VSIDE_WORDS + 16, m = 0u - ((incl >> r) & 1u);
+        u32 carry = 0;
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const u64 t = (u64)acc[i] + (zs[i] & m) + carry;
+            acc[i] = (u32)t;
+            carry = (u32)(t >> 32);
+        }
+        acc[8] += carry;
+    }
+    sc_reduce512(es, acc);
+    sc_recode_window(es);
+    ge_p3 R;
+    ge_identity(R);
+#pragma unroll 1
+    for (int j = 63; j >= -1; j--) {
+        const bool has_b = j >= 0 && (j & 3) == 0 && j < 32;
+        const int nadd = j < 0 ? 0 : j < 33 ? 2 * K : K;
+        const int last = j < 0 ? 3 : 4 + nadd + (has_b ? 2 : 0);
+#pragma unroll 1
+        for (int stp = (j == 63 ? 4 : 0); stp < last; stp++) {
+            const int step = stp < 4 ? stp : stp < 4 + nadd ? 4 : stp == 4 + nadd ? 6 : 7;
+            EDG_VERIFY_STEP(R, step, stp >= 3 && stp + 1 < last, EDG_VBATCH_CACHED, EDG_VLOOP_BASE)
+        }
+    }
+    return fe_is_zero(R.X) & fe_eq(R.Y, R.Z);
 }
 
 EDG_HD u32 ed25519_verify_op(const u32 *sig, const u32 *pub, const uint8_t *msg, u64 len, u32 *state, const u32 *wtab, bool full_scalars = false,
